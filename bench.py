@@ -18,6 +18,9 @@ Beside the headline the line carries the other BASELINE configurations as blocks
                    ranks, ONE all_reduce(MIN) inside the timed region
   move_scoring     config 5: 1,000,000 candidate moves on a 10k-node live snapshot (~300k running pods), moves partitioned
                    contiguously over the ranks, one all_reduce(MAX) + one all_gather of the per-rank top-k
+--dump-outputs DIR writes what the last timed step left for its caller (rank 0): DIR/out_node.npy (the node of every pod of
+the list, -1 = unschedulable) and the per-node totals of simon_state_download (DIR/req_mcpu.npy, ...), as float32 / float64.
+The inputs are generated from fixed seeds, so two builds run with the same arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -204,6 +207,18 @@ def run_reference(args):
             "config": workload_config(args, c0), "cpu_baseline": cb,
             "e2e": {"value": value, "unit": "decisions/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     print(json.dumps(line), flush=True)
+
+
+def dump_outputs(out_dir, eng):
+    """Placements and per-node totals on the device after the last replay, converted exactly (node indices < 2^24 in
+    float32, int64 totals < 2^53 in float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"out_node": eng.results(), **eng.state()}
+    for name, a in arrays.items():
+        f = a.astype(np.float32 if a.dtype == np.int32 else np.float64)
+        if not np.array_equal(f.astype(a.dtype), a):
+            raise ValueError(f"{name} is not exact in {f.dtype}")
+        np.save(os.path.join(out_dir, f"{name}.npy"), f)
 
 
 def workload_config(args, c):
@@ -451,7 +466,10 @@ def main():
     ap.add_argument("--cpu-threads", type=int, default=0, help="host threads of the CPU port (0 = fastest count on this box, capped at 64)")
     ap.add_argument("--no-batch", action="store_true")
     ap.add_argument("--no-blocks", action="store_true", help="headline only: skip the c2 / batch / capacity_search / move_scoring blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "gpu" else args.warmup
 
     if args.impl == "reference":
@@ -504,6 +522,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_max = float(t.item())
     value = world * D * args.steps / (ms_max * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng)
 
     # ---- e2e: host buffers -> C ABI -> host results ----
     import ctypes as C

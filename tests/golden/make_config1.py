@@ -1,7 +1,8 @@
-"""BASELINE config 1 from the reference's own input files (run HERE, where /root/reference exists):
+"""BASELINE config 1 from the reference's own input files, stored in tests/golden/example/ (a verbatim copy of the
+open-simulator project's example/ inputs used here, Apache-2.0):
 
-    cluster  /root/reference/example/cluster/demo_1           (example/simon-config.yaml:12-14 customConfig)
-    apps     /root/reference/example/application/{simple,complicate,more_pods,gpushare}
+    cluster  example/cluster/demo_1           (example/simon-config.yaml:12-14 customConfig)
+    apps     example/application/{simple,complicate,more_pods,gpushare}
              (the non-chart apps of example/simon-config.yaml:20-33 + the GPU-share example; open_local needs the
               Open-Local plugin, which is out of scope, and the yoda chart needs Helm rendering)
 
@@ -12,7 +13,7 @@ reference text) are stored in tests/golden/config1_<name>.npz together with
     * the facts the reference itself pins for such runs (pkg/simulator/core_test.go:364-591): the number of unscheduled
       pods and the pod count per workload.
 tests/test_config1.py replays the stored columns through the oracle (CPU suite) and through the CUDA engine (-m gpu);
-when /root/reference is present it also re-derives the columns from the YAML and checks that nothing drifted.
+it also re-derives the columns from the YAML and checks that nothing drifted.
 
     python tests/golden/make_config1.py
 """
@@ -28,7 +29,7 @@ for p in (os.path.join(ROOT, "open-simulator_b200"), ROOT, os.path.join(ROOT, "t
     if p not in sys.path:
         sys.path.insert(0, p)
 
-REF = "/root/reference/example"
+REF = os.path.join(HERE, "example")
 CASES = {
     "simple": ["simple"],
     "complicate": ["complicate"],

@@ -128,11 +128,10 @@ def test_auto_add_nodes_sweep_and_bisect_agree():
     assert all(sweep.per_k[q]["n_unscheduled"] == 0 for q in range(k, 25))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/example"), reason="reference tree not present (GPU box)")
 def test_apply_config_of_the_reference_example(tmp_path):
     """example/simon-config.yaml with `customConfig: example/cluster/demo_1` (the shipped file points at a developer's
     kubeConfig, SURVEY 8d C1) and the non-chart, non-open-local apps: the 4-node demo cluster cannot hold them, the search
-    reports how many copies of example/newnode/demo_1 are needed."""
+    reports how many copies of example/newnode/demo_1 are needed.  The example inputs are stored in tests/golden/example/."""
     import yaml
     from simon_b200 import apply as A
     cfg = {"apiVersion": "simon/v1alpha1", "kind": "Config", "metadata": {"name": "simon-config"},
@@ -143,7 +142,8 @@ def test_apply_config_of_the_reference_example(tmp_path):
                     "newNode": "example/newnode/demo_1"}}
     path = tmp_path / "simon-config.yaml"
     path.write_text(yaml.safe_dump(cfg))
-    cluster, apps, new_node = A.load_config(str(path), base_dir="/root/reference")
+    base = os.path.join(ROOT, "tests", "golden")
+    cluster, apps, new_node = A.load_config(str(path), base_dir=base)
     assert len(cluster.Nodes) == 4 and len(apps) == 3 and new_node["metadata"]["name"] == "node-1"
     res = A.auto_add_nodes(cluster, apps, new_node, _oracle_factory, kmax=32, method="bisect")
     assert res.unscheduled_without_new_nodes > 0
@@ -152,7 +152,7 @@ def test_apply_config_of_the_reference_example(tmp_path):
     assert sweep.new_node_num == res.new_node_num
     # the shipped config itself is refused for what it is (kubeConfig of a developer machine / Helm chart), not ignored
     with pytest.raises(NotImplementedError):
-        A.load_config("/root/reference/example/simon-config.yaml", base_dir="/root/reference")
+        A.load_config(os.path.join(base, "example", "simon-config.yaml"), base_dir=base)
 
 
 @pytest.mark.gpu

@@ -7,7 +7,7 @@ the native path is asserted here at three levels:
     hand-derived Simon KAT pins) on a sweep of quantity strings, incl. the inf.Dec fallbacks and the error cases;
   * the compiled columns: every array and dimension of simon_snapshot / simon_podset, node order, pod order and identity, for
     synthetic clusters (C2 / C3 shapes, 40 random feature mixes with DaemonSets, GPU share, images), the hand-derived plugin KATs,
-    the DaemonSet cluster and - where /root/reference exists - the reference's own example cluster + applications (config 1);
+    the DaemonSet cluster and the reference's own example cluster + applications (config 1, stored in tests/golden/example/);
   * (-m gpu) simulator.Simulate: simon_host_simulate == simon_b200.simulator.Simulate: per-node pod lists in placement order and
     every UnscheduledPod reason string.
 """
@@ -141,7 +141,6 @@ def test_native_columns_match_python_on_the_daemonset_cluster():
     assert _diff(*T._cluster()) == []
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/example"), reason="reference tree not present (GPU box)")
 @pytest.mark.parametrize("case", ["simple", "complicate", "more_pods", "gpushare", "config_sequence"])
 def test_native_compiles_the_reference_example_inputs_to_the_stored_columns(case):
     """BASELINE config 1: example/cluster/demo_1 x example/application/* through the NATIVE compiler == the columns stored in
