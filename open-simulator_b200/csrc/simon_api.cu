@@ -14,6 +14,7 @@
 
 #include "simon_kernel.cu"   // single translation unit: kernel + host API
 #include "simon_moves.cu"    // candidate-move scoring kernels (config 5)
+#include "simon_drain.cu"    // node-drain fork kernels
 
 namespace {
 
@@ -115,6 +116,10 @@ struct ScenBatch {
     DevBuf<simon_scenario_result> results;
     std::vector<uint32_t> h_order;
     std::vector<int32_t> h_rank;
+    // drains: per chunk the evicted lists (list_off / list_pods), their results by list position, the pods to release
+    DevBuf<uint64_t> list_off;
+    DevBuf<uint32_t> list_pods, list_fail, list_fail_pod, rm_pods, rm_scen;
+    DevBuf<int32_t> list_node, rm_node, live_node;
 };
 
 // satisfyResourceSetting's sums (pkg/apply/apply.go:747-757) per scenario over its active nodes, plus the scenario's counters
@@ -201,6 +206,13 @@ struct simon_ctx {
     // multi-scenario state
     std::vector<ScenState *> scen_states;
     ScenBatch *batch = nullptr;
+    // the live state: pods [0, live_next) placed in order since the last reset (UINT32_MAX: a partial or out-of-order run)
+    uint32_t live_next = 0;
+    std::vector<int32_t> h_pod_fixed, h_pod_guard;   // host copies of the pod columns (pod_fixed_node as given, guard per pod)
+    std::vector<uint8_t> h_pod_pinned;               // per pod: class is SIMON_CLS_PINNED
+    // results of the last simon_drain_run, per evicted pod (simon_drain_download)
+    std::vector<uint32_t> dr_pod, dr_fail;
+    std::vector<int32_t> dr_node;
 };
 
 namespace {
@@ -310,6 +322,14 @@ sk_kernel_fn pick_kernel(uint32_t TPB, uint32_t npt, bool prof) {
     }
     if (prof) return npt == 1 ? simon_prof_kernel_256_1 : npt == 2 ? simon_prof_kernel_256_2 : npt == 3 ? simon_prof_kernel_256_3 : npt == 4 ? simon_prof_kernel_256_4 : simon_prof_kernel_256_0;
     return npt == 1 ? simon_place_kernel_256_1 : npt == 2 ? simon_place_kernel_256_2 : npt == 3 ? simon_place_kernel_256_3 : npt == 4 ? simon_place_kernel_256_4 : simon_place_kernel_256_0;
+}
+
+// the pod-list (drain) variant for (threads per CTA, node slots per thread); nullptr: none
+sk_kernel_fn pick_list_kernel(uint32_t TPB, uint32_t npt) {
+    if (TPB > 384) return nullptr;
+    if (TPB > 320) return npt == 1 ? simon_list_kernel_384_1 : npt == 2 ? simon_list_kernel_384_2 : npt == 3 ? simon_list_kernel_384_3 : simon_list_kernel_384_0;
+    if (TPB > 256) return npt == 1 ? simon_list_kernel_320_1 : npt == 2 ? simon_list_kernel_320_2 : npt == 3 ? simon_list_kernel_320_3 : npt == 4 ? simon_list_kernel_320_4 : simon_list_kernel_320_0;
+    return npt == 1 ? simon_list_kernel_256_1 : npt == 2 ? simon_list_kernel_256_2 : npt == 3 ? simon_list_kernel_256_3 : npt == 4 ? simon_list_kernel_256_4 : simon_list_kernel_256_0;
 }
 
 // clusters of `cs` CTAs x `t` threads with `smem` bytes each that the device holds at once (GPC boundaries included)
@@ -463,14 +483,18 @@ int choose_geometry(simon_ctx *ctx, uint32_t n_active, uint32_t &CS, uint32_t &T
 
 static_assert(sizeof(SkScenario) % 8 == 0, "SkScenario is copied in 8-byte words");
 
-int launch(simon_ctx *ctx, SkParams &P, uint32_t n_scen, uint32_t CS, uint32_t TPB, size_t smem, bool record = true) {
+int launch(simon_ctx *ctx, SkParams &P, uint32_t n_scen, uint32_t CS, uint32_t TPB, size_t smem, bool record = true, bool list = false) {
     sk_kernel_fn fn;
     const uint32_t npt = P.npt;
     if (TPB > SIMON_MAX_TPB) return fail(ctx, SIMON_ERR_LIMIT, "threads per CTA must be <= %u", SIMON_MAX_TPB);
+    if (list && ctx->big) return fail(ctx, SIMON_ERR_LIMIT, "drains of clusters that need the large-cluster kernel variant are not supported");
     // SIMON_PROFILE=1 selects the variants with per-phase clock64 timers (simon_stats cycles); the default variants
     // carry no timers
     static const bool prof = getenv("SIMON_PROFILE") != nullptr;
-    if (ctx->big) {
+    if (list) {
+        fn = pick_list_kernel(TPB, npt);
+        if (!fn) return fail(ctx, SIMON_ERR_LIMIT, "no pod-list kernel variant for %u threads per CTA", TPB);
+    } else if (ctx->big) {
         CU(ctx->d_gnode.alloc(ctx->gnode_stride * (size_t)n_scen * CS));
         P.gnode = ctx->d_gnode.p; P.gnode_stride = ctx->gnode_stride;
         fn = simon_place_kernel_big;
@@ -521,6 +545,70 @@ int launch_range(simon_ctx *ctx, SkParams &P, uint32_t CS, uint32_t TPB, size_t 
         if (rc) return rc;
     }
     if (record) CU(cudaEventRecord(ctx->ev1, ctx->stream));
+    return SIMON_OK;
+}
+
+// Pooled state of a batch of n scenarios (simon_scenarios_run, simon_drain_run): the node lists validated on the host and uploaded in
+// ONE copy each (scenario order and its inverse), one allocation per column with a slot per scenario (contents left as they are:
+// the caller fills them), and the scenario descriptors in h.  `base`: index of scen[0] in the caller's list (error messages).
+int scen_pool_prepare(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, uint32_t base, bool with_out_node, uint32_t &max_active,
+                      std::vector<SkScenario> &h) {
+    cudaStream_t st = ctx->stream;
+    const uint32_t N = ctx->N, N1 = std::max(1u, N), K1 = ctx->K ? ctx->K : 1, P1 = std::max(1u, ctx->n_pods);
+    const size_t cntw = std::max<uint64_t>(1, ctx->cnt_words), nct = std::max(1u, ctx->n_counters), ncl = std::max(1u, ctx->n_classes);
+    if (!ctx->batch) { ctx->batch = new (std::nothrow) ScenBatch(); if (!ctx->batch) return SIMON_ERR_NOMEM; }
+    ScenBatch &B = *ctx->batch;
+    max_active = 0;
+    B.h_order.assign((size_t)n * N1, 0u);
+    B.h_rank.assign((size_t)n * N1, -1);
+    std::vector<uint8_t> ident(n, 0);
+    for (uint32_t i = 0; i < n; i++) {
+        if (scen[i].n_nodes > N) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: too many nodes", base + i);
+        if (scen[i].n_nodes && !scen[i].nodes) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: bad node list", base + i);
+        uint32_t *ord = B.h_order.data() + (size_t)i * N1;
+        int32_t *rank = B.h_rank.data() + (size_t)i * N1;
+        bool id = scen[i].n_nodes == N;
+        for (uint32_t r = 0; r < scen[i].n_nodes; r++) {
+            uint32_t g = scen[i].nodes[r];
+            if (g >= N || rank[g] != -1) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: bad node list", base + i);
+            rank[g] = (int32_t)r;
+            ord[r] = g;
+            if (g != r) id = false;
+        }
+        ident[i] = id ? 1 : 0;
+        max_active = std::max(max_active, scen[i].n_nodes);
+    }
+    CU(B.req_mcpu.alloc((size_t)n * N1)); CU(B.req_mem.alloc((size_t)n * N1)); CU(B.req_eph.alloc((size_t)n * N1));
+    CU(B.nz_mcpu.alloc((size_t)n * N1)); CU(B.nz_mem.alloc((size_t)n * N1)); CU(B.req_scalar.alloc((size_t)n * K1 * N1));
+    CU(B.gpu_used.alloc((size_t)n * SIMON_MAX_GPU_DEV * N1)); CU(B.num_pods.alloc((size_t)n * N1));
+    CU(B.cnt.alloc((size_t)n * cntw)); CU(B.cnt_total.alloc((size_t)n * nct));
+    const size_t tabw = (size_t)SK_MAX_SOFT * ctx->max_dom;
+    CU(B.tp.alloc((size_t)n * tabw)); CU(B.fcount.alloc((size_t)n * tabw)); CU(B.size.alloc((size_t)n * SK_MAX_SOFT));
+    CU(B.hard_reg.alloc((size_t)n * SK_MAX_HARD * ctx->max_dom));
+    CU(B.csum.alloc((size_t)n * ncl * SK_CSUM_W)); CU(B.fbits.alloc((size_t)n * ncl * N1)); CU(B.ocache.alloc((size_t)n * ncl * N1));
+    if (with_out_node) CU(B.out_node.alloc((size_t)n * P1));
+    CU(B.counters.alloc((size_t)n * 2)); CU(B.clk.alloc((size_t)n * 2));
+    CU(B.order.alloc((size_t)n * N1)); CU(B.rank_of.alloc((size_t)n * N1)); CU(B.results.alloc(n));
+    CU(cudaMemcpyAsync(B.order.p, B.h_order.data(), 4ull * n * N1, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(B.rank_of.p, B.h_rank.data(), 4ull * n * N1, cudaMemcpyHostToDevice, st));
+    h.assign(n, SkScenario());
+    for (uint32_t i = 0; i < n; i++) {
+        SkScenario &o = h[i];
+        memset(&o, 0, sizeof(o));
+        o.order = ident[i] ? nullptr : B.order.p + (size_t)i * N1;
+        o.rank_of = ident[i] ? nullptr : B.rank_of.p + (size_t)i * N1;
+        o.n_active = scen[i].n_nodes;
+        o.req_mcpu = B.req_mcpu.p + (size_t)i * N1; o.req_mem = B.req_mem.p + (size_t)i * N1; o.req_eph = B.req_eph.p + (size_t)i * N1;
+        o.nz_mcpu = B.nz_mcpu.p + (size_t)i * N1; o.nz_mem = B.nz_mem.p + (size_t)i * N1;
+        o.req_scalar = B.req_scalar.p + (size_t)i * K1 * N1; o.gpu_used = B.gpu_used.p + (size_t)i * SIMON_MAX_GPU_DEV * N1;
+        o.num_pods = B.num_pods.p + (size_t)i * N1; o.cnt = B.cnt.p + (size_t)i * cntw; o.cnt_total = B.cnt_total.p + (size_t)i * nct;
+        o.tp = B.tp.p + (size_t)i * tabw; o.fcount = B.fcount.p + (size_t)i * tabw; o.size = B.size.p + (size_t)i * SK_MAX_SOFT;
+        o.hard_reg = B.hard_reg.p + (size_t)i * SK_MAX_HARD * ctx->max_dom;
+        o.csum = B.csum.p + (size_t)i * ncl * SK_CSUM_W; o.fbits = B.fbits.p + (size_t)i * ncl * N1; o.ocache = B.ocache.p + (size_t)i * ncl * N1;
+        o.out_node = with_out_node ? B.out_node.p + (size_t)i * P1 : nullptr; o.out_score = nullptr; o.out_gpu = nullptr;
+        o.fail_counts = nullptr; o.fail_pod = nullptr; o.n_fail = B.counters.p + 2ull * i; o.n_sched = B.counters.p + 2ull * i + 1;
+        o.clk = B.clk.p + 2ull * i;
+    }
     return SIMON_OK;
 }
 
@@ -758,6 +846,12 @@ int simon_pods_upload(simon_ctx *ctx, const simon_podset *p) {
     if (rc) return rc;
     rc = reset_state(ctx, ctx->st);
     if (rc) return rc;
+    ctx->live_next = 0;
+    ctx->h_pod_fixed.assign(p->pod_fixed_node, p->pod_fixed_node + p->n_pods);
+    ctx->h_pod_guard.assign(guard.begin(), guard.begin() + p->n_pods);
+    ctx->h_pod_pinned.assign(p->n_pods, 0);
+    for (uint32_t i = 0; i < p->n_pods; i++)
+        ctx->h_pod_pinned[i] = (p->class_blob[p->class_off[p->pod_class[i]] + SCW_FLAGS] & SIMON_CLS_PINNED) ? 1 : 0;
     CU(ctx->d_scen.alloc(1));
     ctx->n_sigs = std::max(1u, p->n_static_sigs);
     {
@@ -779,6 +873,7 @@ int simon_pods_upload(simon_ctx *ctx, const simon_podset *p) {
 int simon_state_reset(simon_ctx *ctx) {
     if (!ctx || !ctx->have_pods) return ctx ? fail(ctx, SIMON_ERR_STATE, "no pods uploaded") : SIMON_ERR_INVALID;
     CU(cudaSetDevice(ctx->device));
+    ctx->live_next = 0;
     int rc = reset_state(ctx, ctx->st);
     if (rc) return rc;
     CU(cudaStreamSynchronize(ctx->stream));
@@ -821,10 +916,13 @@ int simon_schedule(simon_ctx *ctx, uint32_t first, uint32_t count, int32_t *out_
         CU(cudaMemsetAsync(ctx->d_dump_total.p, 0xff, 8ull * std::max(1u, ctx->N), st));     // -1: node not scored (infeasible)
         CU(cudaMemsetAsync(ctx->d_dump_code.p, 0, 4ull * std::max(1u, ctx->N), st));
     }
+    const uint32_t live_after = first == ctx->live_next ? first + count : UINT32_MAX;
+    ctx->live_next = UINT32_MAX;
     rc = launch_range(ctx, P, CS, TPB, smem, first, count, true);
     if (rc) return rc;
     cudaError_t e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) return fail(ctx, SIMON_ERR_CUDA, "kernel failed: %s", cudaGetErrorString(e));
+    ctx->live_next = live_after;
     CU(cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1));
     uint32_t counters[2] = {0, 0};
     CU(cudaMemcpy(counters, ctx->st.counters.p, 8, cudaMemcpyDeviceToHost));
@@ -853,6 +951,7 @@ int simon_replay(simon_ctx *ctx, uint32_t steps, float *out_ms_total) {
     fill_params(ctx, P);
     P.first = 0; P.count = ctx->n_pods; P.max_fail = ctx->max_fail; P.npt = NPT; P.scen = ctx->d_scen.p;
     CU(cudaEventRecord(ctx->ev0, st));
+    if (steps) ctx->live_next = UINT32_MAX;
     for (uint32_t s = 0; s < steps; s++) {
         rc = reset_state(ctx, ctx->st);
         if (rc) return rc;
@@ -864,6 +963,7 @@ int simon_replay(simon_ctx *ctx, uint32_t steps, float *out_ms_total) {
     CU(cudaEventRecord(ctx->ev1, st));
     cudaError_t e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) return fail(ctx, SIMON_ERR_CUDA, "kernel failed: %s", cudaGetErrorString(e));
+    if (steps) ctx->live_next = ctx->n_pods;     // every pass ends with all pods placed
     CU(cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1));
     if (out_ms_total) *out_ms_total = ctx->last_ms;
     return SIMON_OK;
@@ -899,43 +999,13 @@ int simon_scenarios_run(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, 
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     if (n == 0) return SIMON_OK;
-    const uint32_t N = ctx->N, N1 = std::max(1u, N), K1 = ctx->K ? ctx->K : 1, P = ctx->n_pods, P1 = std::max(1u, P);
+    const uint32_t N = ctx->N, N1 = std::max(1u, N), K1 = ctx->K ? ctx->K : 1, P = ctx->n_pods;
     const size_t cntw = std::max<uint64_t>(1, ctx->cnt_words), nct = std::max(1u, ctx->n_counters), ncl = std::max(1u, ctx->n_classes);
-    if (!ctx->batch) { ctx->batch = new (std::nothrow) ScenBatch(); if (!ctx->batch) return SIMON_ERR_NOMEM; }
-    ScenBatch &B = *ctx->batch;
-    // ---- node lists: validated on the host, uploaded in ONE copy each (scenario order and its inverse) ----
     uint32_t max_active = 0;
-    B.h_order.assign((size_t)n * N1, 0u);
-    B.h_rank.assign((size_t)n * N1, -1);
-    std::vector<uint8_t> ident(n, 0);
-    for (uint32_t i = 0; i < n; i++) {
-        if (scen[i].n_nodes > N) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: too many nodes", i);
-        uint32_t *ord = B.h_order.data() + (size_t)i * N1;
-        int32_t *rank = B.h_rank.data() + (size_t)i * N1;
-        bool id = scen[i].n_nodes == N;
-        for (uint32_t r = 0; r < scen[i].n_nodes; r++) {
-            uint32_t g = scen[i].nodes[r];
-            if (g >= N || rank[g] != -1) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: bad node list", i);
-            rank[g] = (int32_t)r;
-            ord[r] = g;
-            if (g != r) id = false;
-        }
-        ident[i] = id ? 1 : 0;
-        max_active = std::max(max_active, scen[i].n_nodes);
-    }
-    // ---- pooled state of all scenarios: one allocation and one memset per column ----
-    CU(B.req_mcpu.alloc((size_t)n * N1)); CU(B.req_mem.alloc((size_t)n * N1)); CU(B.req_eph.alloc((size_t)n * N1));
-    CU(B.nz_mcpu.alloc((size_t)n * N1)); CU(B.nz_mem.alloc((size_t)n * N1)); CU(B.req_scalar.alloc((size_t)n * K1 * N1));
-    CU(B.gpu_used.alloc((size_t)n * SIMON_MAX_GPU_DEV * N1)); CU(B.num_pods.alloc((size_t)n * N1));
-    CU(B.cnt.alloc((size_t)n * cntw)); CU(B.cnt_total.alloc((size_t)n * nct));
-    const size_t tabw = (size_t)SK_MAX_SOFT * ctx->max_dom;
-    CU(B.tp.alloc((size_t)n * tabw)); CU(B.fcount.alloc((size_t)n * tabw)); CU(B.size.alloc((size_t)n * SK_MAX_SOFT));
-    CU(B.hard_reg.alloc((size_t)n * SK_MAX_HARD * ctx->max_dom));
-    CU(B.csum.alloc((size_t)n * ncl * SK_CSUM_W)); CU(B.fbits.alloc((size_t)n * ncl * N1)); CU(B.ocache.alloc((size_t)n * ncl * N1));
-    CU(B.out_node.alloc((size_t)n * P1)); CU(B.counters.alloc((size_t)n * 2)); CU(B.clk.alloc((size_t)n * 2));
-    CU(B.order.alloc((size_t)n * N1)); CU(B.rank_of.alloc((size_t)n * N1)); CU(B.results.alloc(n));
-    CU(cudaMemcpyAsync(B.order.p, B.h_order.data(), 4ull * n * N1, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(B.rank_of.p, B.h_rank.data(), 4ull * n * N1, cudaMemcpyHostToDevice, st));
+    std::vector<SkScenario> h;
+    int rc = scen_pool_prepare(ctx, scen, n, 0, true, max_active, h);
+    if (rc) return rc;
+    ScenBatch &B = *ctx->batch;
     CU(cudaMemsetAsync(B.req_mcpu.p, 0, 8ull * n * N1, st)); CU(cudaMemsetAsync(B.req_mem.p, 0, 8ull * n * N1, st));
     CU(cudaMemsetAsync(B.req_eph.p, 0, 8ull * n * N1, st)); CU(cudaMemsetAsync(B.nz_mcpu.p, 0, 8ull * n * N1, st));
     CU(cudaMemsetAsync(B.nz_mem.p, 0, 8ull * n * N1, st)); CU(cudaMemsetAsync(B.req_scalar.p, 0, 8ull * n * K1 * N1, st));
@@ -945,28 +1015,10 @@ int simon_scenarios_run(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, 
     // call (another node list!); fbits are only read under a valid summary record
     CU(cudaMemsetAsync(B.csum.p, 0, 8ull * n * ncl * SK_CSUM_W, st)); CU(cudaMemsetAsync(B.ocache.p, 0, 8ull * n * ncl * N1, st));
     CU(cudaMemsetAsync(B.counters.p, 0, 8ull * n, st)); CU(cudaMemsetAsync(B.clk.p, 0, 16ull * n, st));
-    std::vector<SkScenario> h(n);
-    for (uint32_t i = 0; i < n; i++) {
-        SkScenario &o = h[i];
-        memset(&o, 0, sizeof(o));
-        o.order = ident[i] ? nullptr : B.order.p + (size_t)i * N1;
-        o.rank_of = ident[i] ? nullptr : B.rank_of.p + (size_t)i * N1;
-        o.n_active = scen[i].n_nodes;
-        o.req_mcpu = B.req_mcpu.p + (size_t)i * N1; o.req_mem = B.req_mem.p + (size_t)i * N1; o.req_eph = B.req_eph.p + (size_t)i * N1;
-        o.nz_mcpu = B.nz_mcpu.p + (size_t)i * N1; o.nz_mem = B.nz_mem.p + (size_t)i * N1;
-        o.req_scalar = B.req_scalar.p + (size_t)i * K1 * N1; o.gpu_used = B.gpu_used.p + (size_t)i * SIMON_MAX_GPU_DEV * N1;
-        o.num_pods = B.num_pods.p + (size_t)i * N1; o.cnt = B.cnt.p + (size_t)i * cntw; o.cnt_total = B.cnt_total.p + (size_t)i * nct;
-        o.tp = B.tp.p + (size_t)i * tabw; o.fcount = B.fcount.p + (size_t)i * tabw; o.size = B.size.p + (size_t)i * SK_MAX_SOFT;
-        o.hard_reg = B.hard_reg.p + (size_t)i * SK_MAX_HARD * ctx->max_dom;
-        o.csum = B.csum.p + (size_t)i * ncl * SK_CSUM_W; o.fbits = B.fbits.p + (size_t)i * ncl * N1; o.ocache = B.ocache.p + (size_t)i * ncl * N1;
-        o.out_node = B.out_node.p + (size_t)i * P1; o.out_score = nullptr; o.out_gpu = nullptr;
-        o.fail_counts = nullptr; o.fail_pod = nullptr; o.n_fail = B.counters.p + 2ull * i; o.n_sched = B.counters.p + 2ull * i + 1;
-        o.clk = B.clk.p + 2ull * i;
-    }
     CU(ctx->d_scen.upload(h.data(), n, st));
     uint32_t CS, TPB, NPT;
     size_t smem;
-    int rc = choose_geometry(ctx, max_active, CS, TPB, NPT, smem, n);
+    rc = choose_geometry(ctx, max_active, CS, TPB, NPT, smem, n);
     if (rc) return rc;
     SkParams Pm;
     fill_params(ctx, Pm);
@@ -981,6 +1033,206 @@ int simon_scenarios_run(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, 
     cudaError_t e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) return fail(ctx, SIMON_ERR_CUDA, "kernel failed: %s", cudaGetErrorString(e));
     CU(cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1));
+    return SIMON_OK;
+}
+
+// ---- node drains (include/simon_gpu.h, "node drains") ------------------------------------------------------------------------
+int simon_drain_run(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, simon_drain_result *out, uint64_t *out_off) {
+    if (!ctx || !out_off || (n && (!scen || !out))) return SIMON_ERR_INVALID;
+    if (!ctx->have_pods) return fail(ctx, SIMON_ERR_STATE, "simon_drain_run before uploads");
+    if (ctx->live_next != ctx->n_pods)
+        return fail(ctx, SIMON_ERR_STATE, "simon_drain_run needs the live state: every pod placed in order by simon_schedule since the last reset");
+    CU(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const uint32_t N = ctx->N, N1 = std::max(1u, N), K1 = ctx->K ? ctx->K : 1, P = ctx->n_pods;
+    const size_t cntw = std::max<uint64_t>(1, ctx->cnt_words), nct = std::max(1u, ctx->n_counters), ncl = std::max(1u, ctx->n_classes);
+    const size_t NFC = SIMON_N_FAIL_CODES;
+    ctx->dr_pod.clear(); ctx->dr_node.clear(); ctx->dr_fail.clear();
+    out_off[0] = 0;
+    ctx->last_ms = 0.f;
+    if (n == 0) return SIMON_OK;
+    // ---- validate every node list before any device work ----
+    uint32_t max_active = 0;
+    {
+        std::vector<uint32_t> seen(N1, 0u);
+        for (uint32_t i = 0; i < n; i++) {
+            if (scen[i].n_nodes > N || (scen[i].n_nodes && !scen[i].nodes)) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: bad node list", i);
+            for (uint32_t r = 0; r < scen[i].n_nodes; r++) {
+                const uint32_t g = scen[i].nodes[r];
+                if (g >= N || seen[g] == i + 1) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: bad node list", i);
+                seen[g] = i + 1;
+            }
+            max_active = std::max(max_active, scen[i].n_nodes);
+        }
+    }
+    // ---- the live placement (downloaded once) as pods per node, ascending pod index ----
+    std::vector<int32_t> live(std::max(1u, P));
+    if (P) CU(cudaMemcpy(live.data(), ctx->st.out_node.p, 4ull * P, cudaMemcpyDeviceToHost));
+    std::vector<uint32_t> node_first(N1 + 1, 0u), node_pods;
+    for (uint32_t p = 0; p < P; p++) if (live[p] >= 0 && (uint32_t)live[p] < N) node_first[live[p] + 1]++;
+    for (uint32_t g = 0; g < N1; g++) node_first[g + 1] += node_first[g];
+    node_pods.resize(std::max(1u, node_first[N1]));
+    {
+        std::vector<uint32_t> fill(node_first.begin(), node_first.end() - 1);
+        for (uint32_t p = 0; p < P; p++) if (live[p] >= 0 && (uint32_t)live[p] < N) node_pods[fill[live[p]]++] = p;
+    }
+    // ---- geometry and chunk size: the pooled state of one scenario, bounded by free device memory ----
+    const size_t tabw = (size_t)SK_MAX_SOFT * ctx->max_dom;
+    const size_t per_scen = (size_t)N1 * (8 * 5 + 8 * K1 + 8 * SIMON_MAX_GPU_DEV + 4 + 8) + 4 * (cntw + nct) + 8 * tabw + 4 * SK_MAX_SOFT +
+                            SK_MAX_HARD * (size_t)ctx->max_dom + ncl * (8 * SK_CSUM_W + 9 * (size_t)N1) + 64 + sizeof(simon_scenario_result);
+    uint32_t chunk = n;
+    {
+        size_t free_b = 0, total_b = 0;
+        CU(cudaMemGetInfo(&free_b, &total_b));
+        size_t avail = free_b;
+        cudaMemPool_t pool;
+        if (cudaDeviceGetDefaultMemPool(&pool, ctx->device) == cudaSuccess) {       // freed blocks stay cached in the pool
+            unsigned long long reserved = 0, used = 0;
+            if (cudaMemPoolGetAttribute(pool, cudaMemPoolAttrReservedMemCurrent, &reserved) == cudaSuccess &&
+                cudaMemPoolGetAttribute(pool, cudaMemPoolAttrUsedMemCurrent, &used) == cudaSuccess && reserved > used)
+                avail += (size_t)(reserved - used);
+        }
+        if (ctx->batch) avail += (ctx->batch->req_mcpu.cap / N1) * per_scen;     // this pool's own slots are reallocated
+        const size_t fit = std::max<size_t>(1, (avail / 10 * 7) / per_scen);
+        chunk = (uint32_t)std::min<size_t>(n, fit);
+    }
+    uint32_t CS, TPB, NPT;
+    size_t smem;
+    int rc = choose_geometry(ctx, max_active, CS, TPB, NPT, smem, chunk);
+    if (rc) return rc;
+    if (ctx->big) return fail(ctx, SIMON_ERR_LIMIT, "drains of clusters that need the large-cluster kernel variant (%u survivors) are not supported", max_active);
+    {
+        sk_kernel_fn fn = pick_list_kernel(TPB, NPT);
+        const int resident = fn ? max_active_clusters(fn, CS, TPB, smem) : 0;
+        if (resident > 0 && chunk > (uint32_t)resident) chunk -= chunk % (uint32_t)resident;      // whole waves of co-resident clusters
+        const char *env = getenv("SIMON_DRAIN_CHUNK");         // forced chunk size (tests: results must not depend on it)
+        if (env && atoi(env) > 0) chunk = std::min<uint32_t>(n, (uint32_t)atoi(env));
+    }
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device);
+    float kernel_ms = 0.f;
+    std::vector<SkScenario> h;
+    std::vector<uint64_t> loff;
+    std::vector<uint32_t> lpods, rm_pods, rm_scen, n_daemon, n_bound, fail_pod, fail_rows;
+    std::vector<int32_t> rm_node, lnode;
+    std::vector<simon_scenario_result> res;
+    for (uint32_t b = 0; b < n; b += chunk) {
+        const uint32_t m = std::min(chunk, n - b);
+        uint32_t ma = 0;
+        rc = scen_pool_prepare(ctx, scen + b, m, b, false, ma, h);
+        if (rc) return rc;
+        ScenBatch &B = *ctx->batch;
+        // ---- classify the pods of every scenario's drained nodes (B.h_rank: -1 = drained) ----
+        loff.assign(m + 1, 0); lpods.clear(); rm_pods.clear(); rm_node.clear(); rm_scen.clear();
+        n_daemon.assign(m, 0); n_bound.assign(m, 0);
+        std::vector<uint32_t> on_d;
+        for (uint32_t i = 0; i < m; i++) {
+            const int32_t *rank = B.h_rank.data() + (size_t)i * N1;
+            on_d.clear();
+            for (uint32_t g = 0; g < N; g++)
+                if (rank[g] < 0) on_d.insert(on_d.end(), node_pods.begin() + node_first[g], node_pods.begin() + node_first[g + 1]);
+            std::sort(on_d.begin(), on_d.end());
+            for (uint32_t q : on_d) {
+                rm_pods.push_back(q); rm_node.push_back(live[q]); rm_scen.push_back(i);
+                if (ctx->h_pod_pinned[q] || ctx->h_pod_guard[q] >= 0) n_daemon[i]++;
+                else if (ctx->h_pod_fixed[q] >= 0) n_bound[i]++;
+                else lpods.push_back(q);
+            }
+            loff[i + 1] = lpods.size();
+        }
+        const size_t tot = lpods.size();
+        lpods.push_back(0);        // padding: the kernel prefetches one entry of an empty list
+        CU(B.list_off.upload(loff.data(), m + 1, st)); CU(B.list_pods.upload(lpods.data(), tot + 1, st));
+        CU(B.list_node.alloc(tot + 1)); CU(B.list_fail.alloc((tot + 1) * NFC)); CU(B.list_fail_pod.alloc(tot + 1));
+        CU(cudaMemsetAsync(B.list_fail.p, 0, 4ull * (tot + 1) * NFC, st));
+        const uint32_t n_rm = (uint32_t)rm_pods.size();
+        CU(B.rm_pods.upload(rm_pods.data(), n_rm, st)); CU(B.rm_node.upload(rm_node.data(), n_rm, st)); CU(B.rm_scen.upload(rm_scen.data(), n_rm, st));
+        for (uint32_t i = 0; i < m; i++) {
+            h[i].out_node = B.list_node.p + loff[i];
+            h[i].fail_counts = B.list_fail.p + loff[i] * NFC;
+            h[i].fail_pod = B.list_fail_pod.p + loff[i];
+        }
+        // the fork starts from the live state: no stored class summary or own-score cache carries over
+        CU(cudaMemsetAsync(B.csum.p, 0, 8ull * m * ncl * SK_CSUM_W, st)); CU(cudaMemsetAsync(B.ocache.p, 0, 8ull * m * ncl * N1, st));
+        CU(cudaMemsetAsync(B.counters.p, 0, 8ull * m, st)); CU(cudaMemsetAsync(B.clk.p, 0, 16ull * m, st));
+        CU(ctx->d_scen.upload(h.data(), m, st));
+        SkParams Pm;
+        fill_params(ctx, Pm);
+        Pm.first = 0; Pm.count = 0; Pm.max_fail = 0xffffffffu; Pm.npt = NPT; Pm.scen = ctx->d_scen.p;
+        Pm.list_off = B.list_off.p; Pm.list_pods = B.list_pods.p;
+        // ---- fork: broadcast the live columns, release the drained pods' counter increments ----
+        SdFork F;
+        memset(&F, 0, sizeof(F));
+        const ScenState &L = ctx->st;
+        auto seg = [&](const void *src, void *dst, uint64_t words, uint64_t stride) {
+            F.seg[F.n_seg++] = SdSegment{(const uint32_t *)src, (uint32_t *)dst, words, stride};
+        };
+        seg(L.req_mcpu.p, B.req_mcpu.p, 2ull * N, 2ull * N1); seg(L.req_mem.p, B.req_mem.p, 2ull * N, 2ull * N1);
+        seg(L.req_eph.p, B.req_eph.p, 2ull * N, 2ull * N1); seg(L.nz_mcpu.p, B.nz_mcpu.p, 2ull * N, 2ull * N1);
+        seg(L.nz_mem.p, B.nz_mem.p, 2ull * N, 2ull * N1); seg(L.req_scalar.p, B.req_scalar.p, 2ull * K1 * N, 2ull * K1 * N1);
+        seg(L.gpu_used.p, B.gpu_used.p, 2ull * SIMON_MAX_GPU_DEV * N, 2ull * SIMON_MAX_GPU_DEV * N1); seg(L.num_pods.p, B.num_pods.p, N, N1);
+        seg(L.cnt.p, B.cnt.p, ctx->cnt_words, cntw); seg(L.cnt_total.p, B.cnt_total.p, ctx->n_counters, nct);
+        F.n_scen = m;
+        uint64_t maxw = 1;
+        for (uint32_t q = 0; q < F.n_seg; q++) maxw = std::max<uint64_t>(maxw, F.seg[q].words);
+        simon_drain_bcast<<<dim3((uint32_t)std::min<uint64_t>((maxw + 255) / 256, (uint64_t)sms * 8), F.n_seg), 256, 0, st>>>(F);
+        CU(cudaGetLastError());
+        ctx->launches++;
+        if (n_rm) {
+            simon_drain_release<<<std::min<uint32_t>((n_rm + 255) / 256, (uint32_t)sms * 8), 256, 0, st>>>(Pm, B.rm_pods.p, B.rm_node.p, B.rm_scen.p, n_rm);
+            CU(cudaGetLastError());
+            ctx->launches++;
+        }
+        // ---- re-place every scenario's evicted pods on its survivors, then the sums over the survivors ----
+        rc = launch(ctx, Pm, m, CS, TPB, smem, true, true);
+        if (rc) return rc;
+        simon_scen_reduce<<<m, 256, 0, st>>>(ctx->d_scen.p, ctx->d_alloc_mcpu.p, ctx->d_alloc_mem.p, B.results.p);
+        CU(cudaGetLastError());
+        res.resize(m);
+        lnode.resize(tot + 1); fail_pod.resize(tot + 1); fail_rows.resize((tot + 1) * NFC);
+        CU(cudaMemcpyAsync(res.data(), B.results.p, sizeof(simon_scenario_result) * m, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(lnode.data(), B.list_node.p, 4ull * tot, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(fail_pod.data(), B.list_fail_pod.p, 4ull * tot, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(fail_rows.data(), B.list_fail.p, 4ull * tot * NFC, cudaMemcpyDeviceToHost, st));
+        cudaError_t e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) return fail(ctx, SIMON_ERR_CUDA, "drain kernels failed: %s", cudaGetErrorString(e));
+        float ms = 0.f;
+        CU(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+        kernel_ms += ms;
+        // ---- results by scenario; failure records (in order of failure) go to their pod's position ----
+        const size_t gbase = ctx->dr_pod.size();
+        ctx->dr_pod.insert(ctx->dr_pod.end(), lpods.begin(), lpods.begin() + tot);
+        ctx->dr_node.insert(ctx->dr_node.end(), lnode.begin(), lnode.begin() + tot);
+        ctx->dr_fail.resize((gbase + tot) * NFC, 0u);
+        for (uint32_t i = 0; i < m; i++) {
+            const simon_scenario_result &r = res[i];
+            const uint64_t len = loff[i + 1] - loff[i];
+            if ((uint64_t)r.n_unscheduled + r.n_scheduled != len)
+                return fail(ctx, SIMON_ERR_CUDA, "scenario %u: %u + %u results for %llu evicted pods", b + i, r.n_unscheduled, r.n_scheduled, (unsigned long long)len);
+            for (uint32_t j = 0; j < r.n_unscheduled; j++) {
+                const uint32_t pos = fail_pod[loff[i] + j];
+                if (pos >= len) return fail(ctx, SIMON_ERR_CUDA, "scenario %u: bad failure record", b + i);
+                memcpy(&ctx->dr_fail[(gbase + loff[i] + pos) * NFC], &fail_rows[(loff[i] + j) * NFC], 4 * NFC);
+            }
+            simon_drain_result &o = out[b + i];
+            memset(&o, 0, sizeof(o));
+            o.n_evicted = (uint32_t)len; o.n_rescheduled = r.n_scheduled; o.n_unscheduled = r.n_unscheduled;
+            o.n_daemon = n_daemon[i]; o.n_bound = n_bound[i];
+            o.req_mcpu = r.req_mcpu; o.alloc_mcpu = r.alloc_mcpu; o.req_mem = r.req_mem; o.alloc_mem = r.alloc_mem;
+            o.elapsed_ms = r.elapsed_ms;
+            out_off[b + i + 1] = out_off[b + i] + len;
+        }
+    }
+    ctx->last_ms = kernel_ms;
+    return SIMON_OK;
+}
+
+int simon_drain_download(simon_ctx *ctx, uint32_t *out_pod, int32_t *out_node, uint32_t *out_fail_counts) {
+    if (!ctx) return SIMON_ERR_INVALID;
+    const size_t n = ctx->dr_pod.size();
+    if (out_pod && n) memcpy(out_pod, ctx->dr_pod.data(), 4 * n);
+    if (out_node && n) memcpy(out_node, ctx->dr_node.data(), 4 * n);
+    if (out_fail_counts && n) memcpy(out_fail_counts, ctx->dr_fail.data(), 4 * n * SIMON_N_FAIL_CODES);
     return SIMON_OK;
 }
 

@@ -112,6 +112,10 @@ struct SkParams {
     long long *dump_total;         // [N]
     int32_t *dump_code;            // [N] 0 = feasible, else the reason bitmask
     unsigned long long *scache;    // [n_sigs][N] packed {st_code, flags, tt, 0, na:int32}
+    // pod-list variants (LIST, drains): scenario s places pods list_pods[list_off[s] .. list_off[s + 1]) in that order; its
+    // out_node / fail records are indexed by position in the list.  Appended last: the fields above keep their offsets.
+    const uint64_t *list_off;
+    const uint32_t *list_pods;
 };
 
 __host__ __device__ inline size_t sk_align(size_t x) { return (x + 15) & ~(size_t)15; }

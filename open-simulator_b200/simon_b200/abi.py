@@ -53,6 +53,13 @@ class SimonMovesResult(C.Structure):
                 ("kernel_ms", C.c_float), ("reserved", C.c_uint32)]
 
 
+class SimonDrainResult(C.Structure):
+    _fields_ = [("n_evicted", C.c_uint32), ("n_rescheduled", C.c_uint32), ("n_unscheduled", C.c_uint32),
+                ("n_daemon", C.c_uint32), ("n_bound", C.c_uint32), ("reserved", C.c_uint32),
+                ("req_mcpu", C.c_int64), ("alloc_mcpu", C.c_int64), ("req_mem", C.c_int64), ("alloc_mem", C.c_int64),
+                ("elapsed_ms", C.c_float), ("reserved2", C.c_uint32)]
+
+
 MOVE_NOOP, MOVE_NOT_PLACED, MOVE_NOT_MOVABLE, MOVE_BAD_INDEX = 1 << 24, 1 << 25, 1 << 26, 1 << 27
 MOVE_GAIN_BIAS = 1000
 

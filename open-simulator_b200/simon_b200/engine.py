@@ -23,7 +23,8 @@ EXPORTS = ["simon_gpu_version", "simon_ctx_create", "simon_ctx_destroy", "simon_
            "simon_gpu_slots_download", "simon_state_download_ext", "simon_debug_set_dump_pod", "simon_debug_dump_read",
            "simon_moves_upload", "simon_moves_run", "simon_moves_replay", "simon_host_go118_sort",
            "simon_host_last_error", "simon_host_compile", "simon_host_plan_free", "simon_host_plan_columns", "simon_host_plan_describe",
-           "simon_host_simulate", "simon_host_free", "simon_host_quantity_probe", "simon_host_plan_fit_error", "simon_host_capacity_search"]
+           "simon_host_simulate", "simon_host_free", "simon_host_quantity_probe", "simon_host_plan_fit_error", "simon_host_capacity_search",
+           "simon_drain_run", "simon_drain_download"]
 
 
 class EngineUnavailable(RuntimeError):
@@ -83,6 +84,10 @@ def lib():
         L.simon_moves_replay.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_float)]
         L.simon_host_go118_sort.restype = C.c_int
         L.simon_host_go118_sort.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
+        L.simon_drain_run.restype = C.c_int
+        L.simon_drain_run.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]
+        L.simon_drain_download.restype = C.c_int
+        L.simon_drain_download.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     except AttributeError:
         if not os.environ.get("SIMON_GPU_LIB"):       # an experiment library may lack the newer entry points; the shipped one may not
             raise
@@ -267,3 +272,29 @@ class Engine:
         out = [dict(n_unscheduled=r.n_unscheduled, n_scheduled=r.n_scheduled, req_mcpu=r.req_mcpu, alloc_mcpu=r.alloc_mcpu,
                     req_mem=r.req_mem, alloc_mem=r.alloc_mem, elapsed_ms=r.elapsed_ms) for r in res]
         return out, out_node
+
+    def drain(self, scenarios: List[np.ndarray]):
+        """Node drains on the live state (simon_drain_run): scenarios = surviving node indices in their scheduling order
+        (drain.survivor_order).  -> (results, off, pod, node, fail_counts): one dict per scenario (counts and sums over the
+        survivors) and, per evicted pod, scenario s owning entries off[s]:off[s+1]: pod index, new node (-1: unschedulable),
+        failure histogram [n, SIMON_N_FAIL_CODES] (zero for placed pods)."""
+        n = len(scenarios)
+        arr = (abi.SimonScenario * max(n, 1))()
+        keep = []
+        for i, nodes in enumerate(scenarios):
+            a = np.ascontiguousarray(nodes, dtype=np.uint32)
+            keep.append(a)
+            arr[i].n_nodes = len(a)
+            arr[i].nodes = a.ctypes.data
+        res = (abi.SimonDrainResult * max(n, 1))()
+        off = np.zeros(n + 1, np.uint64)
+        self._check(lib().simon_drain_run(self.h, arr, n, res, off.ctypes.data))
+        tot = int(off[-1])
+        pod = np.zeros(max(tot, 1), np.uint32)
+        node = np.zeros(max(tot, 1), np.int32)
+        fc = np.zeros((max(tot, 1), abi.N_FAIL_CODES), np.uint32)
+        self._check(lib().simon_drain_download(self.h, pod.ctypes.data, node.ctypes.data, fc.ctypes.data))
+        out = [dict(n_evicted=r.n_evicted, n_rescheduled=r.n_rescheduled, n_unscheduled=r.n_unscheduled, n_daemon=r.n_daemon,
+                    n_bound=r.n_bound, req_mcpu=r.req_mcpu, alloc_mcpu=r.alloc_mcpu, req_mem=r.req_mem, alloc_mem=r.alloc_mem,
+                    elapsed_ms=r.elapsed_ms) for r in res[:n]]
+        return out, off.astype(np.int64), pod[:tot], node[:tot], fc[:tot]
