@@ -88,31 +88,131 @@ struct DevBuf {
     ~DevBuf() { release(); }
 };
 
-struct ScenState {
-    DevBuf<int64_t> req_mcpu, req_mem, req_eph, nz_mcpu, nz_mem, req_scalar, gpu_used;
-    DevBuf<int32_t> num_pods, cnt, cnt_total, tp, fcount, size;
-    DevBuf<long long> csum;
-    DevBuf<uint8_t> fbits;
-    DevBuf<unsigned long long> ocache;
-    DevBuf<uint8_t> hard_reg;
-    DevBuf<int32_t> out_node;
-    DevBuf<int64_t> out_score;
-    DevBuf<uint32_t> out_gpu;
-    DevBuf<uint32_t> fail_counts, fail_pod, counters;   // counters: [0]=n_fail [1]=n_sched
-    DevBuf<unsigned long long> clk;
-    DevBuf<uint32_t> order;
-    DevBuf<int32_t> rank_of;
+// The per-scenario state the placement kernel reaches through SkScenario: one row per column with its class, element size in
+// bytes and elements per slot (d: the extents of the uploaded cluster, each at least 1).  Columns are laid out in this order,
+// so each class is one contiguous byte range:
+//   STATE    what the scenario has placed: zeroed by a reset, broadcast from the live state by a drain fork (32-bit words)
+//   RESTART  cleared whenever a slot restarts, from empty or from a fork: the own-score cache is keyed by the node's pod count,
+//            and the class summaries describe the node set and order of the run that wrote them (the kernel validates a summary
+//            only against flips of nodes it currently owns).  An incremental simon_schedule keeps them.
+//   ALLOC    zeroed when allocated; read only under a valid csum record
+//   SCRATCH  never cleared
+#define SIMON_STATE_COLUMNS(X)                            \
+    X(req_mcpu,   STATE,   8, d.N1)                       \
+    X(req_mem,    STATE,   8, d.N1)                       \
+    X(req_eph,    STATE,   8, d.N1)                       \
+    X(nz_mcpu,    STATE,   8, d.N1)                       \
+    X(nz_mem,     STATE,   8, d.N1)                       \
+    X(req_scalar, STATE,   8, d.K1 * d.N1)                \
+    X(gpu_used,   STATE,   8, SIMON_MAX_GPU_DEV * d.N1)   \
+    X(num_pods,   STATE,   4, d.N1)                       \
+    X(cnt,        STATE,   4, d.cnt_words)                \
+    X(cnt_total,  STATE,   4, d.n_counters)               \
+    X(csum,       RESTART, 8, d.n_classes * SK_CSUM_W)    \
+    X(ocache,     RESTART, 8, d.n_classes * d.N1)         \
+    X(counters,   RESTART, 4, 2)                          \
+    X(clk,        RESTART, 8, 2)                          \
+    X(fbits,      ALLOC,   1, d.n_classes * d.N1)         \
+    X(tp,         SCRATCH, 4, SK_MAX_SOFT * d.max_dom)    \
+    X(fcount,     SCRATCH, 4, SK_MAX_SOFT * d.max_dom)    \
+    X(size,       SCRATCH, 4, SK_MAX_SOFT)                \
+    X(hard_reg,   SCRATCH, 1, SK_MAX_HARD * d.max_dom)
+
+enum ColClass { CC_STATE, CC_RESTART, CC_ALLOC, CC_SCRATCH, CC_END };
+enum StateCol {
+#define X(name, cls, bytes, count) COL_##name,
+    SIMON_STATE_COLUMNS(X)
+#undef X
+    N_COLS
+};
+constexpr ColClass kColClass[N_COLS] = {
+#define X(name, cls, bytes, count) CC_##cls,
+    SIMON_STATE_COLUMNS(X)
+#undef X
+};
+#define X(name, cls, bytes, count) static_assert(CC_##cls != CC_STATE || bytes % 4 == 0, #name ": the fork copies 32-bit words");
+SIMON_STATE_COLUMNS(X)
+#undef X
+constexpr int class_rows(ColClass k) {
+    int r = 0;
+    for (int c = 0; c < N_COLS; c++) {
+        if (c && kColClass[c] < kColClass[c - 1]) return -1;
+        r += kColClass[c] == k;
+    }
+    return r;
+}
+static_assert(class_rows(CC_STATE) >= 0, "state columns are listed in class order");
+static_assert(class_rows(CC_STATE) <= SD_MAX_SEG, "the drain fork takes one segment per STATE column");
+
+struct StateDims { size_t N1, K1, cnt_words, n_counters, n_classes, max_dom; };
+
+// n slots of the scenario state in one device allocation that only grows.  Column-major: column c holds its n slots back to
+// back and starts on a 256-byte boundary.
+struct StatePool {
+    DevBuf<uint8_t> slab;
+    uint32_t n = 0;
+    size_t per_slot[N_COLS] = {}, off[N_COLS + 1] = {};   // bytes per slot; column offsets (off[N_COLS]: the end)
+
+    cudaError_t prepare(const StateDims &d, uint32_t n_slots, cudaStream_t st) {
+        const size_t sz[N_COLS] = {
+#define X(name, cls, bytes, count) (size_t)(bytes) * (count),
+            SIMON_STATE_COLUMNS(X)
+#undef X
+        };
+        n = n_slots;
+        for (int c = 0; c < N_COLS; c++) {
+            per_slot[c] = sz[c];
+            off[c + 1] = (off[c] + n * per_slot[c] + 255) & ~(size_t)255;
+        }
+        const bool grows = !slab.p || off[N_COLS] > slab.cap;
+        cudaError_t e = slab.alloc(off[N_COLS]);
+        if (e != cudaSuccess || !grows) return e;
+        return zero(CC_ALLOC, CC_ALLOC, st);
+    }
+    size_t slot_bytes() const {
+        size_t b = 0;
+        for (int c = 0; c < N_COLS; c++) b += per_slot[c];
+        return b;
+    }
+    size_t class_begin(int k) const {
+        int c = 0;
+        while (c < N_COLS && kColClass[c] < k) c++;
+        return off[c];
+    }
+    // the columns of classes first..last, all slots, in one memset
+    cudaError_t zero(ColClass first, ColClass last, cudaStream_t st) const {
+        return cudaMemsetAsync(slab.p + class_begin(first), 0, class_begin(last + 1) - class_begin(first), st);
+    }
+    template <typename T>
+    void point(T *&field, StateCol c, uint32_t i) const { field = reinterpret_cast<T *>(slab.p + off[c] + i * per_slot[c]); }
+    // slot i's state pointers; order, rank_of, n_active and the outputs are the caller's
+    SkScenario descriptor(uint32_t i) const {
+        SkScenario o;
+        memset(&o, 0, sizeof(o));
+        point(o.req_mcpu, COL_req_mcpu, i); point(o.req_mem, COL_req_mem, i); point(o.req_eph, COL_req_eph, i);
+        point(o.nz_mcpu, COL_nz_mcpu, i); point(o.nz_mem, COL_nz_mem, i); point(o.req_scalar, COL_req_scalar, i);
+        point(o.gpu_used, COL_gpu_used, i); point(o.num_pods, COL_num_pods, i); point(o.cnt, COL_cnt, i);
+        point(o.cnt_total, COL_cnt_total, i); point(o.csum, COL_csum, i); point(o.ocache, COL_ocache, i);
+        point(o.n_fail, COL_counters, i); o.n_sched = o.n_fail + 1;
+        point(o.clk, COL_clk, i); point(o.fbits, COL_fbits, i);
+        point(o.tp, COL_tp, i); point(o.fcount, COL_fcount, i); point(o.size, COL_size, i); point(o.hard_reg, COL_hard_reg, i);
+        return o;
+    }
+    // the drain fork: every STATE column of `live` (one slot, the same extents) into all n slots
+    void fork_from(const StatePool &live, SdFork &F) const {
+        memset(&F, 0, sizeof(F));
+        for (int c = 0; c < N_COLS && kColClass[c] == CC_STATE; c++)
+            F.seg[F.n_seg++] = SdSegment{(const uint32_t *)(live.slab.p + live.off[c]), (uint32_t *)(slab.p + off[c]), per_slot[c] / 4, per_slot[c] / 4};
+        F.n_scen = n;
+    }
 };
 
 }  // namespace
 
 struct ScenBatch {
-    DevBuf<int64_t> req_mcpu, req_mem, req_eph, nz_mcpu, nz_mem, req_scalar, gpu_used;
-    DevBuf<int32_t> num_pods, cnt, cnt_total, tp, fcount, size, out_node, rank_of;
-    DevBuf<long long> csum;
-    DevBuf<uint8_t> fbits, hard_reg;
-    DevBuf<unsigned long long> ocache, clk;
-    DevBuf<uint32_t> counters, order;
+    StatePool pool;
+    DevBuf<int32_t> out_node, rank_of;
+    DevBuf<uint32_t> order;
     DevBuf<simon_scenario_result> results;
     std::vector<uint32_t> h_order;
     std::vector<int32_t> h_rank;
@@ -197,14 +297,16 @@ struct simon_ctx {
     size_t gnode_stride = 0;
     DevBuf<uint32_t> d_sig_class;       // a class per static signature (dense fill of the static verdict cache)
     bool static_filled = false;
-    // single-scenario state
-    ScenState st;
+    // single-scenario state and its outputs
+    StatePool live;
+    DevBuf<int32_t> d_out_node;
+    DevBuf<int64_t> d_out_score;
+    DevBuf<uint32_t> d_out_gpu, d_fail_counts, d_fail_pod;
     uint32_t max_fail = 0;
     DevBuf<SkScenario> d_scen;
     DevBuf<unsigned long long> d_stats, d_scache;
     uint32_t n_sigs = 1, use_scache = 0, simon32 = 0;
     // multi-scenario state
-    std::vector<ScenState *> scen_states;
     ScenBatch *batch = nullptr;
     // the live state: pods [0, live_next) placed in order since the last reset (UINT32_MAX: a partial or out-of-order run)
     uint32_t live_next = 0;
@@ -233,57 +335,9 @@ int fail(simon_ctx *c, int code, const char *fmt, ...) {
         if (e__ != cudaSuccess) return fail(ctx, SIMON_ERR_CUDA, "%s: %s", #call, cudaGetErrorString(e__)); \
     } while (0)
 
-int alloc_state(simon_ctx *ctx, ScenState &s, uint32_t max_fail, bool scores) {
-    const uint32_t N = ctx->N, K = ctx->K ? ctx->K : 1;
-    CU(s.req_mcpu.alloc(N)); CU(s.req_mem.alloc(N)); CU(s.req_eph.alloc(N)); CU(s.nz_mcpu.alloc(N)); CU(s.nz_mem.alloc(N));
-    CU(s.req_scalar.alloc((size_t)K * N)); CU(s.gpu_used.alloc((size_t)SIMON_MAX_GPU_DEV * N)); CU(s.num_pods.alloc(N));
-    CU(s.cnt.alloc(ctx->cnt_words)); CU(s.cnt_total.alloc(ctx->n_counters));
-    CU(s.tp.alloc((size_t)SK_MAX_SOFT * ctx->max_dom)); CU(s.fcount.alloc((size_t)SK_MAX_SOFT * ctx->max_dom));
-    CU(s.size.alloc(SK_MAX_SOFT)); CU(s.hard_reg.alloc((size_t)SK_MAX_HARD * ctx->max_dom));
-    CU(s.csum.alloc((size_t)ctx->n_classes * SK_CSUM_W));
-    CU(s.fbits.alloc((size_t)ctx->n_classes * N));
-    CU(s.ocache.alloc((size_t)ctx->n_classes * N));
-    CU(cudaMemsetAsync(s.ocache.p, 0, 8ull * std::max<size_t>(1, (size_t)ctx->n_classes * N), ctx->stream));
-    CU(cudaMemsetAsync(s.csum.p, 0, 8ull * std::max<size_t>(1, (size_t)ctx->n_classes * SK_CSUM_W), ctx->stream));
-    CU(cudaMemsetAsync(s.fbits.p, 0, std::max<size_t>(1, (size_t)ctx->n_classes * N), ctx->stream));
-    CU(s.out_node.alloc(ctx->n_pods));
-    if (scores) CU(s.out_score.alloc(ctx->n_pods));
-    CU(s.out_gpu.alloc(ctx->n_pods));
-    CU(s.fail_counts.alloc((size_t)max_fail * SIMON_N_FAIL_CODES)); CU(s.fail_pod.alloc(max_fail)); CU(s.counters.alloc(2));
-    CU(s.clk.alloc(2));
-    return SIMON_OK;
-}
-
-int reset_state(simon_ctx *ctx, ScenState &s) {
-    cudaStream_t st = ctx->stream;
-    const uint32_t N = ctx->N, K = ctx->K ? ctx->K : 1;
-    CU(cudaMemsetAsync(s.req_mcpu.p, 0, 8ull * N, st)); CU(cudaMemsetAsync(s.req_mem.p, 0, 8ull * N, st));
-    CU(cudaMemsetAsync(s.req_eph.p, 0, 8ull * N, st)); CU(cudaMemsetAsync(s.nz_mcpu.p, 0, 8ull * N, st));
-    CU(cudaMemsetAsync(s.nz_mem.p, 0, 8ull * N, st)); CU(cudaMemsetAsync(s.req_scalar.p, 0, 8ull * K * N, st));
-    CU(cudaMemsetAsync(s.gpu_used.p, 0, 8ull * SIMON_MAX_GPU_DEV * N, st)); CU(cudaMemsetAsync(s.num_pods.p, 0, 4ull * N, st));
-    CU(cudaMemsetAsync(s.cnt.p, 0, 4ull * (ctx->cnt_words ? ctx->cnt_words : 1), st));
-    CU(cudaMemsetAsync(s.cnt_total.p, 0, 4ull * (ctx->n_counters ? ctx->n_counters : 1), st));
-    // the own-score cache is keyed by the node's pod count, which restarts with the state
-    if (s.ocache.p) CU(cudaMemsetAsync(s.ocache.p, 0, 8ull * std::max<size_t>(1, (size_t)ctx->n_classes * N), st));
-    // the stored feasible-set summaries (and the feasibility bits they are exact for) describe the node set and order of
-    // the run that wrote them: a state that restarts from empty - possibly with another scenario's node list - must not
-    // inherit them (the kernel validates a summary only against flips of nodes it currently owns)
-    if (s.csum.p) CU(cudaMemsetAsync(s.csum.p, 0, 8ull * std::max<size_t>(1, (size_t)ctx->n_classes * SK_CSUM_W), st));
-    return SIMON_OK;
-}
-
-void fill_scen(simon_ctx *ctx, ScenState &s, SkScenario &o, uint32_t n_active, bool identity) {
-    o.order = identity ? nullptr : s.order.p;
-    o.rank_of = identity ? nullptr : s.rank_of.p;
-    o.n_active = n_active;
-    o.pad = 0;
-    o.req_mcpu = s.req_mcpu.p; o.req_mem = s.req_mem.p; o.req_eph = s.req_eph.p; o.nz_mcpu = s.nz_mcpu.p; o.nz_mem = s.nz_mem.p;
-    o.req_scalar = s.req_scalar.p; o.gpu_used = s.gpu_used.p; o.num_pods = s.num_pods.p; o.cnt = s.cnt.p; o.cnt_total = s.cnt_total.p;
-    o.tp = s.tp.p; o.fcount = s.fcount.p; o.size = s.size.p; o.hard_reg = s.hard_reg.p; o.csum = s.csum.p; o.fbits = s.fbits.p; o.ocache = s.ocache.p;
-    o.out_node = s.out_node.p; o.out_score = s.out_score.p; o.out_gpu = s.out_gpu.p;
-    o.fail_counts = s.fail_counts.p; o.fail_pod = s.fail_pod.p; o.n_fail = s.counters.p; o.n_sched = s.counters.p + 1;
-    o.clk = s.clk.p;
-    (void)ctx;
+StateDims state_dims(const simon_ctx *ctx) {
+    return StateDims{std::max(1u, ctx->N), ctx->K ? ctx->K : 1u, std::max<uint64_t>(1, ctx->cnt_words), std::max(1u, ctx->n_counters),
+                     std::max(1u, ctx->n_classes), ctx->max_dom};
 }
 
 void fill_params(simon_ctx *ctx, SkParams &P) {
@@ -309,27 +363,25 @@ void fill_params(simon_ctx *ctx, SkParams &P) {
 #define SIMON_AUTO_TPB 320u
 
 typedef void (*sk_kernel_fn)(const SkParams);
-// the compiled kernel variant for (threads per CTA, node slots per thread); nullptr: none
-sk_kernel_fn pick_kernel(uint32_t TPB, uint32_t npt, bool prof) {
-    if (TPB > 384) return nullptr;
-    if (TPB > 320) {
-        if (prof) return nullptr;
-        return npt == 1 ? simon_place_kernel_384_1 : npt == 2 ? simon_place_kernel_384_2 : npt == 3 ? simon_place_kernel_384_3 : simon_place_kernel_384_0;
-    }
-    if (TPB > 256) {
-        if (prof) return npt == 1 ? simon_prof_kernel_320_1 : npt == 2 ? simon_prof_kernel_320_2 : npt == 3 ? simon_prof_kernel_320_3 : npt == 4 ? simon_prof_kernel_320_4 : simon_prof_kernel_320_0;
-        return npt == 1 ? simon_place_kernel_320_1 : npt == 2 ? simon_place_kernel_320_2 : npt == 3 ? simon_place_kernel_320_3 : npt == 4 ? simon_place_kernel_320_4 : simon_place_kernel_320_0;
-    }
-    if (prof) return npt == 1 ? simon_prof_kernel_256_1 : npt == 2 ? simon_prof_kernel_256_2 : npt == 3 ? simon_prof_kernel_256_3 : npt == 4 ? simon_prof_kernel_256_4 : simon_prof_kernel_256_0;
-    return npt == 1 ? simon_place_kernel_256_1 : npt == 2 ? simon_place_kernel_256_2 : npt == 3 ? simon_place_kernel_256_3 : npt == 4 ? simon_place_kernel_256_4 : simon_place_kernel_256_0;
-}
+// the compiled kernel variants, one per pair of SIMON_GEOMETRIES (simon_kernel.cu); prof: nullptr where the pair has none
+struct SkVariant { uint32_t threads, slots; sk_kernel_fn place, list, prof; };
+#define SIMON_PROF_FN_0(MAXT, NPTT) nullptr
+#define SIMON_PROF_FN_1(MAXT, NPTT) simon_prof_kernel_##MAXT##_##NPTT
+#define SIMON_VARIANT(MAXT, NPTT, PROF) \
+    {MAXT, NPTT, simon_place_kernel_##MAXT##_##NPTT, simon_list_kernel_##MAXT##_##NPTT, SIMON_PROF_FN_##PROF(MAXT, NPTT)},
+const SkVariant kVariants[] = {SIMON_GEOMETRIES(SIMON_VARIANT)};
 
-// the pod-list (drain) variant for (threads per CTA, node slots per thread); nullptr: none
-sk_kernel_fn pick_list_kernel(uint32_t TPB, uint32_t npt) {
-    if (TPB > 384) return nullptr;
-    if (TPB > 320) return npt == 1 ? simon_list_kernel_384_1 : npt == 2 ? simon_list_kernel_384_2 : npt == 3 ? simon_list_kernel_384_3 : simon_list_kernel_384_0;
-    if (TPB > 256) return npt == 1 ? simon_list_kernel_320_1 : npt == 2 ? simon_list_kernel_320_2 : npt == 3 ? simon_list_kernel_320_3 : npt == 4 ? simon_list_kernel_320_4 : simon_list_kernel_320_0;
-    return npt == 1 ? simon_list_kernel_256_1 : npt == 2 ? simon_list_kernel_256_2 : npt == 3 ? simon_list_kernel_256_3 : npt == 4 ? simon_list_kernel_256_4 : simon_list_kernel_256_0;
+// the variant for TPB threads per CTA (rounded up to 256, 320 or 384; nullptr above) and npt node slots per thread: the exact
+// slot count if compiled, else the one that reads it at run time
+const SkVariant *find_variant(uint32_t TPB, uint32_t npt) {
+    const uint32_t t = TPB <= 256 ? 256 : TPB <= 320 ? 320 : TPB <= 384 ? 384 : 0;
+    const SkVariant *any = nullptr;
+    for (const SkVariant &v : kVariants) {
+        if (v.threads != t) continue;
+        if (v.slots == npt) return &v;
+        if (v.slots == 0) any = &v;
+    }
+    return any;
 }
 
 // clusters of `cs` CTAs x `t` threads with `smem` bytes each that the device holds at once (GPC boundaries included)
@@ -383,9 +435,9 @@ int choose_geometry(simon_ctx *ctx, uint32_t n_active, uint32_t &CS, uint32_t &T
             if (npt > 64) continue;
             const size_t b = sk_smem_bytes(npt * t, ctx->T, ctx->emax, ctx->max_blob_words, cs);
             if (b > (size_t)max_smem) continue;
-            sk_kernel_fn fn = pick_kernel(t, npt, false);
-            if (!fn) continue;
-            const int active = max_active_clusters(fn, cs, t, b);
+            const SkVariant *v = find_variant(t, npt);
+            if (!v) continue;
+            const int active = max_active_clusters(v->place, cs, t, b);
             if (active <= 0) continue;
             const uint32_t waves = (n_scen + (uint32_t)active - 1) / (uint32_t)active;
             const double cost = waves * (380.0 + 162.0 * npt + (t > 320 ? 30.0 : 0.0) + 2.0 * cs);
@@ -485,21 +537,20 @@ static_assert(sizeof(SkScenario) % 8 == 0, "SkScenario is copied in 8-byte words
 
 int launch(simon_ctx *ctx, SkParams &P, uint32_t n_scen, uint32_t CS, uint32_t TPB, size_t smem, bool record = true, bool list = false) {
     sk_kernel_fn fn;
-    const uint32_t npt = P.npt;
     if (TPB > SIMON_MAX_TPB) return fail(ctx, SIMON_ERR_LIMIT, "threads per CTA must be <= %u", SIMON_MAX_TPB);
-    if (list && ctx->big) return fail(ctx, SIMON_ERR_LIMIT, "drains of clusters that need the large-cluster kernel variant are not supported");
     // SIMON_PROFILE=1 selects the variants with per-phase clock64 timers (simon_stats cycles); the default variants
     // carry no timers
     static const bool prof = getenv("SIMON_PROFILE") != nullptr;
+    const SkVariant *v = find_variant(TPB, P.npt);
     if (list) {
-        fn = pick_list_kernel(TPB, npt);
+        fn = v ? v->list : nullptr;
         if (!fn) return fail(ctx, SIMON_ERR_LIMIT, "no pod-list kernel variant for %u threads per CTA", TPB);
     } else if (ctx->big) {
         CU(ctx->d_gnode.alloc(ctx->gnode_stride * (size_t)n_scen * CS));
         P.gnode = ctx->d_gnode.p; P.gnode_stride = ctx->gnode_stride;
         fn = simon_place_kernel_big;
     } else {
-        fn = pick_kernel(TPB, npt, prof);
+        fn = v ? (prof ? v->prof : v->place) : nullptr;
         if (!fn) return fail(ctx, SIMON_ERR_LIMIT, "no kernel variant for %u threads per CTA%s", TPB, prof ? " with phase timers" : "");
     }
     CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -548,67 +599,73 @@ int launch_range(simon_ctx *ctx, SkParams &P, uint32_t CS, uint32_t TPB, size_t 
     return SIMON_OK;
 }
 
-// Pooled state of a batch of n scenarios (simon_scenarios_run, simon_drain_run): the node lists validated on the host and uploaded in
-// ONE copy each (scenario order and its inverse), one allocation per column with a slot per scenario (contents left as they are:
-// the caller fills them), and the scenario descriptors in h.  `base`: index of scen[0] in the caller's list (error messages).
-int scen_pool_prepare(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, uint32_t base, bool with_out_node, uint32_t &max_active,
-                      std::vector<SkScenario> &h) {
+// The setup simon_schedule and simon_replay share: geometry, the live descriptor on the device (every node in index order, the
+// context's outputs) and the launch parameters.
+int live_setup(simon_ctx *ctx, SkParams &P, uint32_t &CS, uint32_t &TPB, size_t &smem) {
+    uint32_t NPT;
+    int rc = choose_geometry(ctx, ctx->N, CS, TPB, NPT, smem);
+    if (rc) return rc;
+    SkScenario sc = ctx->live.descriptor(0);
+    sc.n_active = ctx->N;
+    sc.out_node = ctx->d_out_node.p; sc.out_score = ctx->d_out_score.p; sc.out_gpu = ctx->d_out_gpu.p;
+    sc.fail_counts = ctx->d_fail_counts.p; sc.fail_pod = ctx->d_fail_pod.p;
+    CU(cudaMemcpyAsync(ctx->d_scen.p, &sc, sizeof(sc), cudaMemcpyHostToDevice, ctx->stream));
+    fill_params(ctx, P);
+    P.max_fail = ctx->max_fail; P.npt = NPT; P.scen = ctx->d_scen.p;
+    return SIMON_OK;
+}
+
+// The node lists of a batch (simon_scenarios_run, simon_drain_run), all checked before any device work; max_active: the longest.
+int check_scenarios(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, uint32_t &max_active) {
+    const uint32_t N = ctx->N;
+    std::vector<uint32_t> seen(std::max(1u, N), 0u);
+    max_active = 0;
+    for (uint32_t i = 0; i < n; i++) {
+        if (scen[i].n_nodes > N) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: too many nodes", i);
+        if (scen[i].n_nodes && !scen[i].nodes) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: bad node list", i);
+        for (uint32_t r = 0; r < scen[i].n_nodes; r++) {
+            const uint32_t g = scen[i].nodes[r];
+            if (g >= N || seen[g] == i + 1) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: bad node list", i);
+            seen[g] = i + 1;
+        }
+        max_active = std::max(max_active, scen[i].n_nodes);
+    }
+    return SIMON_OK;
+}
+
+// The batch of n scenarios with checked node lists: scenario order and its inverse uploaded in ONE copy each, n slots of the
+// state pool (contents left as they are: the caller clears or forks them), and the descriptors in h, with out_node per
+// scenario if asked (the other outputs are the caller's).
+int batch_prepare(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, bool with_out_node, std::vector<SkScenario> &h) {
     cudaStream_t st = ctx->stream;
-    const uint32_t N = ctx->N, N1 = std::max(1u, N), K1 = ctx->K ? ctx->K : 1, P1 = std::max(1u, ctx->n_pods);
-    const size_t cntw = std::max<uint64_t>(1, ctx->cnt_words), nct = std::max(1u, ctx->n_counters), ncl = std::max(1u, ctx->n_classes);
+    const uint32_t N = ctx->N, N1 = std::max(1u, N), P1 = std::max(1u, ctx->n_pods);
     if (!ctx->batch) { ctx->batch = new (std::nothrow) ScenBatch(); if (!ctx->batch) return SIMON_ERR_NOMEM; }
     ScenBatch &B = *ctx->batch;
-    max_active = 0;
+    CU(B.pool.prepare(state_dims(ctx), n, st));
+    if (with_out_node) CU(B.out_node.alloc((size_t)n * P1));
+    CU(B.order.alloc((size_t)n * N1)); CU(B.rank_of.alloc((size_t)n * N1)); CU(B.results.alloc(n));
     B.h_order.assign((size_t)n * N1, 0u);
     B.h_rank.assign((size_t)n * N1, -1);
-    std::vector<uint8_t> ident(n, 0);
+    h.resize(n);
     for (uint32_t i = 0; i < n; i++) {
-        if (scen[i].n_nodes > N) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: too many nodes", base + i);
-        if (scen[i].n_nodes && !scen[i].nodes) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: bad node list", base + i);
         uint32_t *ord = B.h_order.data() + (size_t)i * N1;
         int32_t *rank = B.h_rank.data() + (size_t)i * N1;
         bool id = scen[i].n_nodes == N;
         for (uint32_t r = 0; r < scen[i].n_nodes; r++) {
-            uint32_t g = scen[i].nodes[r];
-            if (g >= N || rank[g] != -1) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: bad node list", base + i);
+            const uint32_t g = scen[i].nodes[r];
             rank[g] = (int32_t)r;
             ord[r] = g;
             if (g != r) id = false;
         }
-        ident[i] = id ? 1 : 0;
-        max_active = std::max(max_active, scen[i].n_nodes);
+        SkScenario &o = h[i];
+        o = B.pool.descriptor(i);
+        o.order = id ? nullptr : B.order.p + (size_t)i * N1;
+        o.rank_of = id ? nullptr : B.rank_of.p + (size_t)i * N1;
+        o.n_active = scen[i].n_nodes;
+        o.out_node = with_out_node ? B.out_node.p + (size_t)i * P1 : nullptr;
     }
-    CU(B.req_mcpu.alloc((size_t)n * N1)); CU(B.req_mem.alloc((size_t)n * N1)); CU(B.req_eph.alloc((size_t)n * N1));
-    CU(B.nz_mcpu.alloc((size_t)n * N1)); CU(B.nz_mem.alloc((size_t)n * N1)); CU(B.req_scalar.alloc((size_t)n * K1 * N1));
-    CU(B.gpu_used.alloc((size_t)n * SIMON_MAX_GPU_DEV * N1)); CU(B.num_pods.alloc((size_t)n * N1));
-    CU(B.cnt.alloc((size_t)n * cntw)); CU(B.cnt_total.alloc((size_t)n * nct));
-    const size_t tabw = (size_t)SK_MAX_SOFT * ctx->max_dom;
-    CU(B.tp.alloc((size_t)n * tabw)); CU(B.fcount.alloc((size_t)n * tabw)); CU(B.size.alloc((size_t)n * SK_MAX_SOFT));
-    CU(B.hard_reg.alloc((size_t)n * SK_MAX_HARD * ctx->max_dom));
-    CU(B.csum.alloc((size_t)n * ncl * SK_CSUM_W)); CU(B.fbits.alloc((size_t)n * ncl * N1)); CU(B.ocache.alloc((size_t)n * ncl * N1));
-    if (with_out_node) CU(B.out_node.alloc((size_t)n * P1));
-    CU(B.counters.alloc((size_t)n * 2)); CU(B.clk.alloc((size_t)n * 2));
-    CU(B.order.alloc((size_t)n * N1)); CU(B.rank_of.alloc((size_t)n * N1)); CU(B.results.alloc(n));
     CU(cudaMemcpyAsync(B.order.p, B.h_order.data(), 4ull * n * N1, cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(B.rank_of.p, B.h_rank.data(), 4ull * n * N1, cudaMemcpyHostToDevice, st));
-    h.assign(n, SkScenario());
-    for (uint32_t i = 0; i < n; i++) {
-        SkScenario &o = h[i];
-        memset(&o, 0, sizeof(o));
-        o.order = ident[i] ? nullptr : B.order.p + (size_t)i * N1;
-        o.rank_of = ident[i] ? nullptr : B.rank_of.p + (size_t)i * N1;
-        o.n_active = scen[i].n_nodes;
-        o.req_mcpu = B.req_mcpu.p + (size_t)i * N1; o.req_mem = B.req_mem.p + (size_t)i * N1; o.req_eph = B.req_eph.p + (size_t)i * N1;
-        o.nz_mcpu = B.nz_mcpu.p + (size_t)i * N1; o.nz_mem = B.nz_mem.p + (size_t)i * N1;
-        o.req_scalar = B.req_scalar.p + (size_t)i * K1 * N1; o.gpu_used = B.gpu_used.p + (size_t)i * SIMON_MAX_GPU_DEV * N1;
-        o.num_pods = B.num_pods.p + (size_t)i * N1; o.cnt = B.cnt.p + (size_t)i * cntw; o.cnt_total = B.cnt_total.p + (size_t)i * nct;
-        o.tp = B.tp.p + (size_t)i * tabw; o.fcount = B.fcount.p + (size_t)i * tabw; o.size = B.size.p + (size_t)i * SK_MAX_SOFT;
-        o.hard_reg = B.hard_reg.p + (size_t)i * SK_MAX_HARD * ctx->max_dom;
-        o.csum = B.csum.p + (size_t)i * ncl * SK_CSUM_W; o.fbits = B.fbits.p + (size_t)i * ncl * N1; o.ocache = B.ocache.p + (size_t)i * ncl * N1;
-        o.out_node = with_out_node ? B.out_node.p + (size_t)i * P1 : nullptr; o.out_score = nullptr; o.out_gpu = nullptr;
-        o.fail_counts = nullptr; o.fail_pod = nullptr; o.n_fail = B.counters.p + 2ull * i; o.n_sched = B.counters.p + 2ull * i + 1;
-        o.clk = B.clk.p + 2ull * i;
-    }
     return SIMON_OK;
 }
 
@@ -645,7 +702,6 @@ int simon_ctx_create(const simon_ctx_opts *opts, simon_ctx **out) {
 void simon_ctx_destroy(simon_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
-    for (auto *s : ctx->scen_states) delete s;
     delete ctx->batch;
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
     if (ctx->ev1) cudaEventDestroy(ctx->ev1);
@@ -842,10 +898,12 @@ int simon_pods_upload(simon_ctx *ctx, const simon_podset *p) {
     for (uint32_t i = 0; i < p->n_pods; i++) ctx->bypass[i] = (guard[i] == -2 || p->pod_fixed_node[i] != -1) ? 1 : 0;
     CU(cudaStreamSynchronize(st));
     ctx->max_fail = std::max(1u, p->n_pods);      // every pod of the list may fail: one histogram row each (96 B)
-    int rc = alloc_state(ctx, ctx->st, ctx->max_fail, (ctx->opt_flags & SIMON_OPT_RECORD_SCORES) != 0);
-    if (rc) return rc;
-    rc = reset_state(ctx, ctx->st);
-    if (rc) return rc;
+    CU(ctx->live.prepare(state_dims(ctx), 1, st));
+    CU(ctx->live.zero(CC_STATE, CC_ALLOC, st));
+    CU(ctx->d_out_node.alloc(ctx->n_pods));
+    if (ctx->opt_flags & SIMON_OPT_RECORD_SCORES) CU(ctx->d_out_score.alloc(ctx->n_pods));
+    CU(ctx->d_out_gpu.alloc(ctx->n_pods));
+    CU(ctx->d_fail_counts.alloc((size_t)ctx->max_fail * SIMON_N_FAIL_CODES)); CU(ctx->d_fail_pod.alloc(ctx->max_fail));
     ctx->live_next = 0;
     ctx->h_pod_fixed.assign(p->pod_fixed_node, p->pod_fixed_node + p->n_pods);
     ctx->h_pod_guard.assign(guard.begin(), guard.begin() + p->n_pods);
@@ -874,8 +932,7 @@ int simon_state_reset(simon_ctx *ctx) {
     if (!ctx || !ctx->have_pods) return ctx ? fail(ctx, SIMON_ERR_STATE, "no pods uploaded") : SIMON_ERR_INVALID;
     CU(cudaSetDevice(ctx->device));
     ctx->live_next = 0;
-    int rc = reset_state(ctx, ctx->st);
-    if (rc) return rc;
+    CU(ctx->live.zero(CC_STATE, CC_RESTART, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
     return SIMON_OK;
 }
@@ -884,9 +941,9 @@ int simon_results_download(simon_ctx *ctx, uint32_t first, uint32_t count, int32
     if (!ctx || !ctx->have_pods) return SIMON_ERR_STATE;
     if ((uint64_t)first + count > ctx->n_pods) return fail(ctx, SIMON_ERR_INVALID, "range out of bounds");
     CU(cudaSetDevice(ctx->device));
-    if (out_node) CU(cudaMemcpyAsync(out_node, ctx->st.out_node.p + first, 4ull * count, cudaMemcpyDeviceToHost, ctx->stream));
-    if (out_score && ctx->st.out_score.p)
-        CU(cudaMemcpyAsync(out_score, ctx->st.out_score.p + first, 8ull * count, cudaMemcpyDeviceToHost, ctx->stream));
+    if (out_node) CU(cudaMemcpyAsync(out_node, ctx->d_out_node.p + first, 4ull * count, cudaMemcpyDeviceToHost, ctx->stream));
+    if (out_score && ctx->d_out_score.p)
+        CU(cudaMemcpyAsync(out_score, ctx->d_out_score.p + first, 8ull * count, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
     return SIMON_OK;
 }
@@ -899,18 +956,15 @@ int simon_schedule(simon_ctx *ctx, uint32_t first, uint32_t count, int32_t *out_
     CU(cudaSetDevice(ctx->device));
     if (count == 0) { if (out_n_fail) *out_n_fail = 0; return SIMON_OK; }
     cudaStream_t st = ctx->stream;
-    uint32_t CS, TPB, NPT;
+    uint32_t CS, TPB;
     size_t smem;
-    int rc = choose_geometry(ctx, ctx->N, CS, TPB, NPT, smem);
-    if (rc) return rc;
-    SkScenario sc;
-    fill_scen(ctx, ctx->st, sc, ctx->N, true);
-    CU(cudaMemcpyAsync(ctx->d_scen.p, &sc, sizeof(sc), cudaMemcpyHostToDevice, st));
-    CU(cudaMemsetAsync(ctx->st.fail_counts.p, 0, 4ull * ctx->max_fail * SIMON_N_FAIL_CODES, st));
-    CU(cudaMemsetAsync(ctx->st.counters.p, 0, 8, st));
     SkParams P;
-    fill_params(ctx, P);
-    P.first = first; P.count = count; P.max_fail = ctx->max_fail; P.npt = NPT; P.scen = ctx->d_scen.p;
+    int rc = live_setup(ctx, P, CS, TPB, smem);
+    if (rc) return rc;
+    P.first = first; P.count = count;
+    const SkScenario L = ctx->live.descriptor(0);
+    CU(cudaMemsetAsync(ctx->d_fail_counts.p, 0, 4ull * ctx->max_fail * SIMON_N_FAIL_CODES, st));
+    CU(cudaMemsetAsync(L.n_fail, 0, 8, st));
     if (ctx->dump_pod >= first && ctx->dump_pod < first + count) {
         P.dump_pod = ctx->dump_pod; P.dump_total = ctx->d_dump_total.p; P.dump_code = ctx->d_dump_code.p;
         CU(cudaMemsetAsync(ctx->d_dump_total.p, 0xff, 8ull * std::max(1u, ctx->N), st));     // -1: node not scored (infeasible)
@@ -925,13 +979,13 @@ int simon_schedule(simon_ctx *ctx, uint32_t first, uint32_t count, int32_t *out_
     ctx->live_next = live_after;
     CU(cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1));
     uint32_t counters[2] = {0, 0};
-    CU(cudaMemcpy(counters, ctx->st.counters.p, 8, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(counters, L.n_fail, 8, cudaMemcpyDeviceToHost));
     if (out_n_fail) *out_n_fail = counters[0];
-    if (out_node) CU(cudaMemcpy(out_node, ctx->st.out_node.p + first, 4ull * count, cudaMemcpyDeviceToHost));
-    if (out_score && ctx->st.out_score.p) CU(cudaMemcpy(out_score, ctx->st.out_score.p + first, 8ull * count, cudaMemcpyDeviceToHost));
+    if (out_node) CU(cudaMemcpy(out_node, ctx->d_out_node.p + first, 4ull * count, cudaMemcpyDeviceToHost));
+    if (out_score && ctx->d_out_score.p) CU(cudaMemcpy(out_score, ctx->d_out_score.p + first, 8ull * count, cudaMemcpyDeviceToHost));
     uint32_t nf = std::min(std::min(counters[0], max_fail), ctx->max_fail);
-    if (nf && out_fail_counts) CU(cudaMemcpy(out_fail_counts, ctx->st.fail_counts.p, 4ull * nf * SIMON_N_FAIL_CODES, cudaMemcpyDeviceToHost));
-    if (nf && out_fail_pod) CU(cudaMemcpy(out_fail_pod, ctx->st.fail_pod.p, 4ull * nf, cudaMemcpyDeviceToHost));
+    if (nf && out_fail_counts) CU(cudaMemcpy(out_fail_counts, ctx->d_fail_counts.p, 4ull * nf * SIMON_N_FAIL_CODES, cudaMemcpyDeviceToHost));
+    if (nf && out_fail_pod) CU(cudaMemcpy(out_fail_pod, ctx->d_fail_pod.p, 4ull * nf, cudaMemcpyDeviceToHost));
     return SIMON_OK;
 }
 
@@ -940,23 +994,17 @@ int simon_replay(simon_ctx *ctx, uint32_t steps, float *out_ms_total) {
     if (!ctx->have_pods) return fail(ctx, SIMON_ERR_STATE, "simon_replay before uploads");
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    uint32_t CS, TPB, NPT;
+    uint32_t CS, TPB;
     size_t smem;
-    int rc = choose_geometry(ctx, ctx->N, CS, TPB, NPT, smem);
-    if (rc) return rc;
-    SkScenario sc;
-    fill_scen(ctx, ctx->st, sc, ctx->N, true);
-    CU(cudaMemcpyAsync(ctx->d_scen.p, &sc, sizeof(sc), cudaMemcpyHostToDevice, st));
     SkParams P;
-    fill_params(ctx, P);
-    P.first = 0; P.count = ctx->n_pods; P.max_fail = ctx->max_fail; P.npt = NPT; P.scen = ctx->d_scen.p;
+    int rc = live_setup(ctx, P, CS, TPB, smem);
+    if (rc) return rc;
+    P.first = 0; P.count = ctx->n_pods;
     CU(cudaEventRecord(ctx->ev0, st));
     if (steps) ctx->live_next = UINT32_MAX;
     for (uint32_t s = 0; s < steps; s++) {
-        rc = reset_state(ctx, ctx->st);
-        if (rc) return rc;
-        CU(cudaMemsetAsync(ctx->st.fail_counts.p, 0, 4ull * ctx->max_fail * SIMON_N_FAIL_CODES, st));
-        CU(cudaMemsetAsync(ctx->st.counters.p, 0, 8, st));
+        CU(ctx->live.zero(CC_STATE, CC_RESTART, st));
+        CU(cudaMemsetAsync(ctx->d_fail_counts.p, 0, 4ull * ctx->max_fail * SIMON_N_FAIL_CODES, st));
         rc = launch_range(ctx, P, CS, TPB, smem, 0, ctx->n_pods, false);
         if (rc) return rc;
     }
@@ -984,12 +1032,13 @@ int simon_state_download(simon_ctx *ctx, int64_t *req_mcpu, int64_t *req_mem, in
     if (!ctx || !ctx->have_pods) return SIMON_ERR_STATE;
     CU(cudaSetDevice(ctx->device));
     const uint32_t N = ctx->N;
-    if (req_mcpu) CU(cudaMemcpy(req_mcpu, ctx->st.req_mcpu.p, 8ull * N, cudaMemcpyDeviceToHost));
-    if (req_mem) CU(cudaMemcpy(req_mem, ctx->st.req_mem.p, 8ull * N, cudaMemcpyDeviceToHost));
-    if (req_eph) CU(cudaMemcpy(req_eph, ctx->st.req_eph.p, 8ull * N, cudaMemcpyDeviceToHost));
-    if (nz_mcpu) CU(cudaMemcpy(nz_mcpu, ctx->st.nz_mcpu.p, 8ull * N, cudaMemcpyDeviceToHost));
-    if (nz_mem) CU(cudaMemcpy(nz_mem, ctx->st.nz_mem.p, 8ull * N, cudaMemcpyDeviceToHost));
-    if (num_pods) CU(cudaMemcpy(num_pods, ctx->st.num_pods.p, 4ull * N, cudaMemcpyDeviceToHost));
+    const SkScenario L = ctx->live.descriptor(0);
+    if (req_mcpu) CU(cudaMemcpy(req_mcpu, L.req_mcpu, 8ull * N, cudaMemcpyDeviceToHost));
+    if (req_mem) CU(cudaMemcpy(req_mem, L.req_mem, 8ull * N, cudaMemcpyDeviceToHost));
+    if (req_eph) CU(cudaMemcpy(req_eph, L.req_eph, 8ull * N, cudaMemcpyDeviceToHost));
+    if (nz_mcpu) CU(cudaMemcpy(nz_mcpu, L.nz_mcpu, 8ull * N, cudaMemcpyDeviceToHost));
+    if (nz_mem) CU(cudaMemcpy(nz_mem, L.nz_mem, 8ull * N, cudaMemcpyDeviceToHost));
+    if (num_pods) CU(cudaMemcpy(num_pods, L.num_pods, 4ull * N, cudaMemcpyDeviceToHost));
     return SIMON_OK;
 }
 
@@ -999,22 +1048,15 @@ int simon_scenarios_run(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, 
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     if (n == 0) return SIMON_OK;
-    const uint32_t N = ctx->N, N1 = std::max(1u, N), K1 = ctx->K ? ctx->K : 1, P = ctx->n_pods;
-    const size_t cntw = std::max<uint64_t>(1, ctx->cnt_words), nct = std::max(1u, ctx->n_counters), ncl = std::max(1u, ctx->n_classes);
+    const uint32_t P = ctx->n_pods;
     uint32_t max_active = 0;
+    int rc = check_scenarios(ctx, scen, n, max_active);
+    if (rc) return rc;
     std::vector<SkScenario> h;
-    int rc = scen_pool_prepare(ctx, scen, n, 0, true, max_active, h);
+    rc = batch_prepare(ctx, scen, n, true, h);
     if (rc) return rc;
     ScenBatch &B = *ctx->batch;
-    CU(cudaMemsetAsync(B.req_mcpu.p, 0, 8ull * n * N1, st)); CU(cudaMemsetAsync(B.req_mem.p, 0, 8ull * n * N1, st));
-    CU(cudaMemsetAsync(B.req_eph.p, 0, 8ull * n * N1, st)); CU(cudaMemsetAsync(B.nz_mcpu.p, 0, 8ull * n * N1, st));
-    CU(cudaMemsetAsync(B.nz_mem.p, 0, 8ull * n * N1, st)); CU(cudaMemsetAsync(B.req_scalar.p, 0, 8ull * n * K1 * N1, st));
-    CU(cudaMemsetAsync(B.gpu_used.p, 0, 8ull * n * SIMON_MAX_GPU_DEV * N1, st)); CU(cudaMemsetAsync(B.num_pods.p, 0, 4ull * n * N1, st));
-    CU(cudaMemsetAsync(B.cnt.p, 0, 4ull * n * cntw, st)); CU(cudaMemsetAsync(B.cnt_total.p, 0, 4ull * n * nct, st));
-    // each scenario starts from an empty state: no stored class summary / own-score cache may survive from an earlier
-    // call (another node list!); fbits are only read under a valid summary record
-    CU(cudaMemsetAsync(B.csum.p, 0, 8ull * n * ncl * SK_CSUM_W, st)); CU(cudaMemsetAsync(B.ocache.p, 0, 8ull * n * ncl * N1, st));
-    CU(cudaMemsetAsync(B.counters.p, 0, 8ull * n, st)); CU(cudaMemsetAsync(B.clk.p, 0, 16ull * n, st));
+    CU(B.pool.zero(CC_STATE, CC_RESTART, st));       // each scenario starts from an empty state
     CU(ctx->d_scen.upload(h.data(), n, st));
     uint32_t CS, TPB, NPT;
     size_t smem;
@@ -1044,30 +1086,18 @@ int simon_drain_run(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, simo
         return fail(ctx, SIMON_ERR_STATE, "simon_drain_run needs the live state: every pod placed in order by simon_schedule since the last reset");
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    const uint32_t N = ctx->N, N1 = std::max(1u, N), K1 = ctx->K ? ctx->K : 1, P = ctx->n_pods;
-    const size_t cntw = std::max<uint64_t>(1, ctx->cnt_words), nct = std::max(1u, ctx->n_counters), ncl = std::max(1u, ctx->n_classes);
+    const uint32_t N = ctx->N, N1 = std::max(1u, N), P = ctx->n_pods;
     const size_t NFC = SIMON_N_FAIL_CODES;
     ctx->dr_pod.clear(); ctx->dr_node.clear(); ctx->dr_fail.clear();
     out_off[0] = 0;
     ctx->last_ms = 0.f;
     if (n == 0) return SIMON_OK;
-    // ---- validate every node list before any device work ----
     uint32_t max_active = 0;
-    {
-        std::vector<uint32_t> seen(N1, 0u);
-        for (uint32_t i = 0; i < n; i++) {
-            if (scen[i].n_nodes > N || (scen[i].n_nodes && !scen[i].nodes)) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: bad node list", i);
-            for (uint32_t r = 0; r < scen[i].n_nodes; r++) {
-                const uint32_t g = scen[i].nodes[r];
-                if (g >= N || seen[g] == i + 1) return fail(ctx, SIMON_ERR_INVALID, "scenario %u: bad node list", i);
-                seen[g] = i + 1;
-            }
-            max_active = std::max(max_active, scen[i].n_nodes);
-        }
-    }
+    int rc = check_scenarios(ctx, scen, n, max_active);
+    if (rc) return rc;
     // ---- the live placement (downloaded once) as pods per node, ascending pod index ----
     std::vector<int32_t> live(std::max(1u, P));
-    if (P) CU(cudaMemcpy(live.data(), ctx->st.out_node.p, 4ull * P, cudaMemcpyDeviceToHost));
+    if (P) CU(cudaMemcpy(live.data(), ctx->d_out_node.p, 4ull * P, cudaMemcpyDeviceToHost));
     std::vector<uint32_t> node_first(N1 + 1, 0u), node_pods;
     for (uint32_t p = 0; p < P; p++) if (live[p] >= 0 && (uint32_t)live[p] < N) node_first[live[p] + 1]++;
     for (uint32_t g = 0; g < N1; g++) node_first[g + 1] += node_first[g];
@@ -1076,10 +1106,9 @@ int simon_drain_run(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, simo
         std::vector<uint32_t> fill(node_first.begin(), node_first.end() - 1);
         for (uint32_t p = 0; p < P; p++) if (live[p] >= 0 && (uint32_t)live[p] < N) node_pods[fill[live[p]]++] = p;
     }
-    // ---- geometry and chunk size: the pooled state of one scenario, bounded by free device memory ----
-    const size_t tabw = (size_t)SK_MAX_SOFT * ctx->max_dom;
-    const size_t per_scen = (size_t)N1 * (8 * 5 + 8 * K1 + 8 * SIMON_MAX_GPU_DEV + 4 + 8) + 4 * (cntw + nct) + 8 * tabw + 4 * SK_MAX_SOFT +
-                            SK_MAX_HARD * (size_t)ctx->max_dom + ncl * (8 * SK_CSUM_W + 9 * (size_t)N1) + 64 + sizeof(simon_scenario_result);
+    // ---- geometry and chunk size: the pooled state of one scenario (a slot has the live state's layout), its order and rank
+    // columns and its result, bounded by free device memory ----
+    const size_t per_scen = ctx->live.slot_bytes() + 8ull * N1 + sizeof(simon_scenario_result) + 64;
     uint32_t chunk = n;
     {
         size_t free_b = 0, total_b = 0;
@@ -1092,18 +1121,18 @@ int simon_drain_run(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, simo
                 cudaMemPoolGetAttribute(pool, cudaMemPoolAttrUsedMemCurrent, &used) == cudaSuccess && reserved > used)
                 avail += (size_t)(reserved - used);
         }
-        if (ctx->batch) avail += (ctx->batch->req_mcpu.cap / N1) * per_scen;     // this pool's own slots are reallocated
+        if (ctx->batch) avail += ctx->batch->pool.slab.cap;     // this pool's own slab is reallocated
         const size_t fit = std::max<size_t>(1, (avail / 10 * 7) / per_scen);
         chunk = (uint32_t)std::min<size_t>(n, fit);
     }
     uint32_t CS, TPB, NPT;
     size_t smem;
-    int rc = choose_geometry(ctx, max_active, CS, TPB, NPT, smem, chunk);
+    rc = choose_geometry(ctx, max_active, CS, TPB, NPT, smem, chunk);
     if (rc) return rc;
     if (ctx->big) return fail(ctx, SIMON_ERR_LIMIT, "drains of clusters that need the large-cluster kernel variant (%u survivors) are not supported", max_active);
     {
-        sk_kernel_fn fn = pick_list_kernel(TPB, NPT);
-        const int resident = fn ? max_active_clusters(fn, CS, TPB, smem) : 0;
+        const SkVariant *v = find_variant(TPB, NPT);
+        const int resident = v ? max_active_clusters(v->list, CS, TPB, smem) : 0;
         if (resident > 0 && chunk > (uint32_t)resident) chunk -= chunk % (uint32_t)resident;      // whole waves of co-resident clusters
         const char *env = getenv("SIMON_DRAIN_CHUNK");         // forced chunk size (tests: results must not depend on it)
         if (env && atoi(env) > 0) chunk = std::min<uint32_t>(n, (uint32_t)atoi(env));
@@ -1118,8 +1147,7 @@ int simon_drain_run(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, simo
     std::vector<simon_scenario_result> res;
     for (uint32_t b = 0; b < n; b += chunk) {
         const uint32_t m = std::min(chunk, n - b);
-        uint32_t ma = 0;
-        rc = scen_pool_prepare(ctx, scen + b, m, b, false, ma, h);
+        rc = batch_prepare(ctx, scen + b, m, false, h);
         if (rc) return rc;
         ScenBatch &B = *ctx->batch;
         // ---- classify the pods of every scenario's drained nodes (B.h_rank: -1 = drained) ----
@@ -1152,9 +1180,7 @@ int simon_drain_run(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, simo
             h[i].fail_counts = B.list_fail.p + loff[i] * NFC;
             h[i].fail_pod = B.list_fail_pod.p + loff[i];
         }
-        // the fork starts from the live state: no stored class summary or own-score cache carries over
-        CU(cudaMemsetAsync(B.csum.p, 0, 8ull * m * ncl * SK_CSUM_W, st)); CU(cudaMemsetAsync(B.ocache.p, 0, 8ull * m * ncl * N1, st));
-        CU(cudaMemsetAsync(B.counters.p, 0, 8ull * m, st)); CU(cudaMemsetAsync(B.clk.p, 0, 16ull * m, st));
+        CU(B.pool.zero(CC_RESTART, CC_RESTART, st));        // a forked slot restarts: no cache carries over
         CU(ctx->d_scen.upload(h.data(), m, st));
         SkParams Pm;
         fill_params(ctx, Pm);
@@ -1162,17 +1188,7 @@ int simon_drain_run(simon_ctx *ctx, const simon_scenario *scen, uint32_t n, simo
         Pm.list_off = B.list_off.p; Pm.list_pods = B.list_pods.p;
         // ---- fork: broadcast the live columns, release the drained pods' counter increments ----
         SdFork F;
-        memset(&F, 0, sizeof(F));
-        const ScenState &L = ctx->st;
-        auto seg = [&](const void *src, void *dst, uint64_t words, uint64_t stride) {
-            F.seg[F.n_seg++] = SdSegment{(const uint32_t *)src, (uint32_t *)dst, words, stride};
-        };
-        seg(L.req_mcpu.p, B.req_mcpu.p, 2ull * N, 2ull * N1); seg(L.req_mem.p, B.req_mem.p, 2ull * N, 2ull * N1);
-        seg(L.req_eph.p, B.req_eph.p, 2ull * N, 2ull * N1); seg(L.nz_mcpu.p, B.nz_mcpu.p, 2ull * N, 2ull * N1);
-        seg(L.nz_mem.p, B.nz_mem.p, 2ull * N, 2ull * N1); seg(L.req_scalar.p, B.req_scalar.p, 2ull * K1 * N, 2ull * K1 * N1);
-        seg(L.gpu_used.p, B.gpu_used.p, 2ull * SIMON_MAX_GPU_DEV * N, 2ull * SIMON_MAX_GPU_DEV * N1); seg(L.num_pods.p, B.num_pods.p, N, N1);
-        seg(L.cnt.p, B.cnt.p, ctx->cnt_words, cntw); seg(L.cnt_total.p, B.cnt_total.p, ctx->n_counters, nct);
-        F.n_scen = m;
+        B.pool.fork_from(ctx->live, F);
         uint64_t maxw = 1;
         for (uint32_t q = 0; q < F.n_seg; q++) maxw = std::max<uint64_t>(maxw, F.seg[q].words);
         simon_drain_bcast<<<dim3((uint32_t)std::min<uint64_t>((maxw + 255) / 256, (uint64_t)sms * 8), F.n_seg), 256, 0, st>>>(F);
@@ -1254,7 +1270,7 @@ int simon_gpu_slots_download(simon_ctx *ctx, uint32_t first, uint32_t count, uin
     if (!ctx || !ctx->have_pods || !out_slots) return SIMON_ERR_STATE;
     if ((uint64_t)first + count > ctx->n_pods) return fail(ctx, SIMON_ERR_INVALID, "range out of bounds");
     CU(cudaSetDevice(ctx->device));
-    CU(cudaMemcpy(out_slots, ctx->st.out_gpu.p + first, 4ull * count, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(out_slots, ctx->d_out_gpu.p + first, 4ull * count, cudaMemcpyDeviceToHost));
     return SIMON_OK;
 }
 
@@ -1262,8 +1278,9 @@ int simon_state_download_ext(simon_ctx *ctx, int64_t *req_scalar, int64_t *gpu_u
     if (!ctx || !ctx->have_pods) return SIMON_ERR_STATE;
     CU(cudaSetDevice(ctx->device));
     const uint32_t N = ctx->N;
-    if (req_scalar && ctx->K) CU(cudaMemcpy(req_scalar, ctx->st.req_scalar.p, 8ull * ctx->K * N, cudaMemcpyDeviceToHost));
-    if (gpu_used) CU(cudaMemcpy(gpu_used, ctx->st.gpu_used.p, 8ull * SIMON_MAX_GPU_DEV * N, cudaMemcpyDeviceToHost));
+    const SkScenario L = ctx->live.descriptor(0);
+    if (req_scalar && ctx->K) CU(cudaMemcpy(req_scalar, L.req_scalar, 8ull * ctx->K * N, cudaMemcpyDeviceToHost));
+    if (gpu_used) CU(cudaMemcpy(gpu_used, L.gpu_used, 8ull * SIMON_MAX_GPU_DEV * N, cudaMemcpyDeviceToHost));
     return SIMON_OK;
 }
 
@@ -1271,20 +1288,21 @@ int simon_state_download_ext(simon_ctx *ctx, int64_t *req_scalar, int64_t *gpu_u
 static int moves_launch(simon_ctx *ctx, bool record) {
     cudaStream_t st = ctx->stream;
     const uint32_t N = ctx->N, n = ctx->mv_n;
+    const SkScenario L = ctx->live.descriptor(0);
     if (record) CU(cudaEventRecord(ctx->ev0, st));
     simon_moves_pack<<<std::max(std::max(1u, (N + 255) / 256), std::min(1184u, (ctx->n_pods + 255) / 256)), 256, 0, st>>>(N, ctx->T, ctx->d_alloc_mcpu.p, ctx->d_alloc_mem.p, ctx->d_alloc_eph.p, ctx->d_alloc_pods.p,
-                                                                     ctx->d_topo_dom.p, ctx->st.req_mcpu.p, ctx->st.req_mem.p, ctx->st.req_eph.p,
-                                                                     ctx->st.nz_mcpu.p, ctx->st.nz_mem.p, ctx->st.num_pods.p, ctx->d_mv_nodes.p,
+                                                                     ctx->d_topo_dom.p, L.req_mcpu, L.req_mem, L.req_eph,
+                                                                     L.nz_mcpu, L.nz_mem, L.num_pods, ctx->d_mv_nodes.p,
                                                                      ctx->d_mv_best_pod.p, ctx->n_pods, ctx->d_mv_best.p, ctx->d_mv_hist.p,
-                                                                     ctx->d_pod_class.p, ctx->st.out_node.p, ctx->d_mv_classes.p, ctx->d_mv_pods.p);
+                                                                     ctx->d_pod_class.p, ctx->d_out_node.p, ctx->d_mv_classes.p, ctx->d_mv_pods.p);
     SmvParams P;
     memset(&P, 0, sizeof(P));
     P.N = N; P.K = ctx->K; P.WT = ctx->WT; P.T = ctx->T; P.n_pods = ctx->n_pods; P.n_moves = n; P.use_scache = ctx->use_scache;
-    P.nodes = ctx->d_mv_nodes.p; P.alloc_scalar = ctx->d_alloc_scalar.p; P.req_scalar = ctx->st.req_scalar.p; P.node_flags = ctx->d_node_flags.p;
+    P.nodes = ctx->d_mv_nodes.p; P.alloc_scalar = ctx->d_alloc_scalar.p; P.req_scalar = L.req_scalar; P.node_flags = ctx->d_node_flags.p;
     P.label_bits = ctx->d_label_bits.p; P.taint_hard = ctx->d_taint_hard.p; P.topo_dom = ctx->d_topo_dom.p;
     P.pods = ctx->d_mv_pods.p;
-    P.class_off = ctx->d_class_off.p; P.class_blob = ctx->d_class_blob.p; P.classes = ctx->d_mv_classes.p; P.pod_class = ctx->d_pod_class.p; P.placement = ctx->st.out_node.p;
-    P.cnt = ctx->st.cnt.p; P.cnt_total = ctx->st.cnt_total.p; P.scache = ctx->d_scache.p; P.moves = ctx->d_moves.p;
+    P.class_off = ctx->d_class_off.p; P.class_blob = ctx->d_class_blob.p; P.classes = ctx->d_mv_classes.p; P.pod_class = ctx->d_pod_class.p; P.placement = ctx->d_out_node.p;
+    P.cnt = L.cnt; P.cnt_total = L.cnt_total; P.scache = ctx->d_scache.p; P.moves = ctx->d_moves.p;
     P.out_gain = ctx->d_mv_gain.p; P.out_code = ctx->d_mv_code.p; P.best_per_pod = ctx->d_mv_best_pod.p; P.best_global = ctx->d_mv_best.p;
     P.hist = ctx->d_mv_hist.p; P.move_base = ctx->mv_base;
     if (n) {

@@ -1443,53 +1443,30 @@ extern "C" __global__ void __launch_bounds__(256) simon_import_kernel(const __gr
     }
 }
 
-#define SIMON_KERNEL(MAXT, NPTT)                                                                         \
-    extern "C" __global__ void __launch_bounds__(MAXT, 1) simon_place_kernel_##MAXT##_##NPTT(const __grid_constant__ SkParams P) { \
-        simon_place_body<MAXT, NPTT, false>(P);                                                          \
-    }                                                                                                    \
-    extern "C" __global__ void __launch_bounds__(MAXT, 1) simon_prof_kernel_##MAXT##_##NPTT(const __grid_constant__ SkParams P) { \
-        simon_place_body<MAXT, NPTT, true>(P);                                                           \
-    }
 extern "C" __global__ void __launch_bounds__(320, 1) simon_place_kernel_big(const __grid_constant__ SkParams P) {
     simon_place_body<320, 0, false, true>(P);
 }
-SIMON_KERNEL(256, 0)
-SIMON_KERNEL(256, 1)
-SIMON_KERNEL(256, 2)
-SIMON_KERNEL(256, 3)
-SIMON_KERNEL(256, 4)
-SIMON_KERNEL(320, 0)
-SIMON_KERNEL(320, 1)
-SIMON_KERNEL(320, 2)
-SIMON_KERNEL(320, 3)
-SIMON_KERNEL(320, 4)
-// 384 threads = 12 warps = 3 per SM sub-partition, the same register ceiling (168) as 320 threads: one slot per thread less where the
-// nodes of a CTA fall between the two (scenario batches on 9-CTA clusters: 3 slots instead of 4).  No profiling variants.
-#define SIMON_KERNEL_PLAIN(MAXT, NPTT)                                                                   \
+// The compiled (threads per CTA, node slots per thread) pairs; slots 0 reads the count at run time.  Each pair has a placement
+// kernel simon_place_kernel_T_S and a pod-list kernel simon_list_kernel_T_S (drains, simon_drain.cu); PROF 1 adds the
+// phase-timer variant simon_prof_kernel_T_S.  384 threads = 12 warps = 3 per SM sub-partition, the same register ceiling (168)
+// as 320 threads: one slot per thread less where the nodes of a CTA fall between the two (scenario batches on 9-CTA clusters:
+// 3 slots instead of 4).  simon_api.cu builds its variant table from the same list.
+#define SIMON_GEOMETRIES(X)                                                                        \
+    X(256, 0, 1) X(256, 1, 1) X(256, 2, 1) X(256, 3, 1) X(256, 4, 1)                                \
+    X(320, 0, 1) X(320, 1, 1) X(320, 2, 1) X(320, 3, 1) X(320, 4, 1)                                \
+    X(384, 0, 0) X(384, 1, 0) X(384, 2, 0) X(384, 3, 0)
+
+#define SIMON_PROF_KERNEL_0(MAXT, NPTT)
+#define SIMON_PROF_KERNEL_1(MAXT, NPTT)                                                                  \
+    extern "C" __global__ void __launch_bounds__(MAXT, 1) simon_prof_kernel_##MAXT##_##NPTT(const __grid_constant__ SkParams P) { \
+        simon_place_body<MAXT, NPTT, true>(P);                                                           \
+    }
+#define SIMON_KERNELS(MAXT, NPTT, PROF)                                                                  \
     extern "C" __global__ void __launch_bounds__(MAXT, 1) simon_place_kernel_##MAXT##_##NPTT(const __grid_constant__ SkParams P) { \
         simon_place_body<MAXT, NPTT, false>(P);                                                          \
-    }
-SIMON_KERNEL_PLAIN(384, 0)
-SIMON_KERNEL_PLAIN(384, 1)
-SIMON_KERNEL_PLAIN(384, 2)
-SIMON_KERNEL_PLAIN(384, 3)
-// Pod-list variants (drains, simon_drain.cu): one per (threads, slots) pair the batch geometry can choose; no profiling or
-// large-cluster variant.
-#define SIMON_KERNEL_LIST(MAXT, NPTT)                                                                    \
+    }                                                                                                    \
+    SIMON_PROF_KERNEL_##PROF(MAXT, NPTT)                                                                 \
     extern "C" __global__ void __launch_bounds__(MAXT, 1) simon_list_kernel_##MAXT##_##NPTT(const __grid_constant__ SkParams P) { \
         simon_place_body<MAXT, NPTT, false, false, true>(P);                                             \
     }
-SIMON_KERNEL_LIST(256, 0)
-SIMON_KERNEL_LIST(256, 1)
-SIMON_KERNEL_LIST(256, 2)
-SIMON_KERNEL_LIST(256, 3)
-SIMON_KERNEL_LIST(256, 4)
-SIMON_KERNEL_LIST(320, 0)
-SIMON_KERNEL_LIST(320, 1)
-SIMON_KERNEL_LIST(320, 2)
-SIMON_KERNEL_LIST(320, 3)
-SIMON_KERNEL_LIST(320, 4)
-SIMON_KERNEL_LIST(384, 0)
-SIMON_KERNEL_LIST(384, 1)
-SIMON_KERNEL_LIST(384, 2)
-SIMON_KERNEL_LIST(384, 3)
+SIMON_GEOMETRIES(SIMON_KERNELS)

@@ -255,16 +255,20 @@ class Engine:
         self._check(lib().simon_moves_replay(self.h, steps, C.byref(ms)))
         return float(ms.value)
 
+    @staticmethod
+    def _scenario_array(scenarios: List[np.ndarray]):
+        """The simon_scenario array of node lists, and the uint32 arrays it points into (to be kept alive across the call)."""
+        arr = (abi.SimonScenario * max(len(scenarios), 1))()
+        keep = [np.ascontiguousarray(nodes, dtype=np.uint32) for nodes in scenarios]
+        for i, a in enumerate(keep):
+            arr[i].n_nodes = len(a)
+            arr[i].nodes = a.ctypes.data
+        return arr, keep
+
     def run_scenarios(self, scenarios: List[np.ndarray], want_nodes: bool = False):
         """scenarios: list of uint32 arrays (active node indices in scenario order)."""
         n = len(scenarios)
-        arr = (abi.SimonScenario * n)()
-        keep = []
-        for i, nodes in enumerate(scenarios):
-            a = np.ascontiguousarray(nodes, dtype=np.uint32)
-            keep.append(a)
-            arr[i].n_nodes = len(a)
-            arr[i].nodes = a.ctypes.data
+        arr, keep = self._scenario_array(scenarios)
         res = (abi.SimonScenarioResult * n)()
         P = self.c.pods_dims["n_pods"]
         out_node = np.full((n, P), -9, np.int32) if want_nodes else None
@@ -279,13 +283,7 @@ class Engine:
         survivors) and, per evicted pod, scenario s owning entries off[s]:off[s+1]: pod index, new node (-1: unschedulable),
         failure histogram [n, SIMON_N_FAIL_CODES] (zero for placed pods)."""
         n = len(scenarios)
-        arr = (abi.SimonScenario * max(n, 1))()
-        keep = []
-        for i, nodes in enumerate(scenarios):
-            a = np.ascontiguousarray(nodes, dtype=np.uint32)
-            keep.append(a)
-            arr[i].n_nodes = len(a)
-            arr[i].nodes = a.ctypes.data
+        arr, keep = self._scenario_array(scenarios)
         res = (abi.SimonDrainResult * max(n, 1))()
         off = np.zeros(n + 1, np.uint64)
         self._check(lib().simon_drain_run(self.h, arr, n, res, off.ctypes.data))
